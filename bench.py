@@ -37,6 +37,12 @@ Every result is compared with the CPU oracle's answer for the exact workload
 
 `--impl reference` times the reference's CPU implementation of the same query
 (oracle/_ref = the reference's own dna.c when it could be compiled, else the oracle port).
+
+`--dump-outputs DIR` writes what the timed legs returned in their last step as DIR/<name>.npy (float64), so that
+two builds can be compared output for output (the inputs are generated from fixed seeds):
+  stats         total, distinct, unique of the resident-input leg (c5: one row k, total, distinct, unique per k)
+  stats_e2e     the same from the host-buffer leg
+  extract_rows  a fixed, seeded sample of the extraction leg's rows: row index, high and low 32 bits of the k-mer
 """
 import argparse
 import ctypes as C
@@ -78,6 +84,17 @@ def measured_peaks():
             return float(json.load(f)["hbm_gbs"]), "measured"
     except Exception:
         return 6650.0, "fallback"
+
+
+DUMP_ROWS = 1 << 20  # rows of the extraction leg sampled by --dump-outputs (at most 24 MB as float64)
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: one DIR/<name>.npy per array, as float64 (every value dumped is below 2**53, so exact)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def golden(name):
@@ -244,6 +261,8 @@ def run_reference(args):
         _, dt, stats, kind, sample_used = cpu_reference_rate(n_bases, k, seed, threads, sample, reads)
         wall += dt
         total += stats[0]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"stats": stats})
     value = total / wall / 1e9
     sample_desc = (f"first {sample_used} bases of the workload per step, {REF_WHAT[kind]}, {threads} threads "
                    "(Postgres itself would run this serially: generate_kmers is PARALLEL UNSAFE; the hash table of a "
@@ -297,6 +316,7 @@ def run_sweep(args, ctx, torch, dev, stream, peak, peak_src):
     assert ctx.lib.dnagpu_seq_download(ctx.handle, seq.handle, C.c_void_p(host.data_ptr()), seq.n_words) == 0
     ks = list(range(3, 33))
     per_k, total_rows, total_ms, launches = {}, 0, 0.0, 0
+    dumped = {"stats": [], "stats_e2e": []}
     sampler = ClockSampler(dev.index)
     sampler.start()
     for k in ks:
@@ -316,9 +336,12 @@ def run_sweep(args, ctx, torch, dev, stream, peak, peak_src):
         ms = e0.elapsed_time(e1) / args.steps
         g = golden(f"c5_k{k}") if not args.n_bases else None
         res = (st.total, st.distinct, st.unique)
+        dumped["stats"].append((k,) + res)
         if g is not None and res != (g["total"], g["distinct"], g["unique"]):
             print(f"bench: k={k}: result {res} differs from the oracle's {(g['total'], g['distinct'], g['unique'])}: "
                   "no line printed", file=sys.stderr)
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, {"stats": dumped["stats"]})
             return 1
         method = ("dense" if any(n.startswith("count_dense") for n in kernels) else
                   "partition" if "count_buckets" in kernels else "hash")
@@ -330,8 +353,11 @@ def run_sweep(args, ctx, torch, dev, stream, peak, peak_src):
     clocks = sampler.stop()
     t0 = time.perf_counter()
     for k in ks:  # the host-buffer call for every k: 250 MB H2D each
-        ctx.count_kmers_ptr(C.c_void_p(host.data_ptr()), n_bases, k)
+        st = ctx.count_kmers_ptr(C.c_void_p(host.data_ptr()), n_bases, k)
+        dumped["stats_e2e"].append((k, st.total, st.distinct, st.unique))
     e2e_s = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dumped)
     slow = max(per_k, key=lambda q: per_k[q]["ms"])
     cpu, one = cpu_baselines(n_bases, 31, seed, None, args.cpu_sample, 1_000_000)
     # roofline of the slowest k: the partition pipeline moves 0.25 B/base + 8 + 16 + 8 B per k-mer (DESIGN.md 4)
@@ -360,7 +386,7 @@ def run_sweep(args, ctx, torch, dev, stream, peak, peak_src):
 
 
 def run_b200(args):
-    import numpy as np  # noqa: F401
+    import numpy as np
     import torch
     import torch.distributed as dist
     import dnagpu
@@ -540,7 +566,7 @@ def run_b200(args):
             ring2.close()
 
         # ---- extraction GB/s (the second half of the metric), timed on its own ----
-        extract = None
+        extract, extract_rows = None, None
         if not args.no_extract and not reads and n_bases >= 1_000_000:
             xs_bases = min(local_bases, 1_000_000_000)
             xs = ctx.synth_range(n_bases, seed, REPEAT_EVERY, first, max(0, xs_bases - k + 1), k)
@@ -551,16 +577,20 @@ def run_b200(args):
             x0, x1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             torch.cuda.synchronize(dev)
             x0.record(stream)
-            xn = 10
+            xn = args.steps
             for _ in range(xn):
                 ctx.extract(xs, k, out=xout)
             x1.record(stream)
             torch.cuda.synchronize(dev)
             xms = x0.elapsed_time(x1) / xn
+            if args.dump_outputs:
+                idx = np.unique(np.random.default_rng(0).integers(0, xr, size=min(xr, DUMP_ROWS)))
+                rows = xout[torch.from_numpy(idx).to(dev)].cpu().numpy().view(np.uint64)
+                extract_rows = np.stack([idx, rows >> 32, rows & 0xFFFFFFFF], axis=1)
             xbytes = 0.25 * xs_bases + 8.0 * xr
             extract = {"rows": xr, "ms": xms, "gkmer_s": xr / xms / 1e6, "gbs": xbytes / xms / 1e6,
                        "frac": xbytes / xms / 1e6 / peak, "bytes_per_row": 8.25,
-                       "note": "output (8 B/row) larger than L2; 10 back-to-back launches"}
+                       "note": f"output (8 B/row) larger than L2; {xn} back-to-back launches"}
             # ... and the WHERE clause over those materialised rows (kmer ^@ 'AC': 1/16 of them pass), rows kept in order
             from dnagpu import _where
             fw, _keep = _where("AC", None)
@@ -593,6 +623,9 @@ def run_b200(args):
         t = torch.tensor([ms, e2e_s], dtype=torch.float64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms, e2e_s = t.tolist()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"stats": stats, "stats_e2e": stats_e2e,
+                                         **({"extract_rows": extract_rows} if extract_rows is not None else {})})
     assert reads or stats[0] == n_rows_total, (stats, n_rows_total)
     assert tuple(stats) == tuple(stats_e2e), (stats, stats_e2e)
     # parity gate: the CPU oracle's answer for this exact workload (tests/golden/big_expected.json, produced by
@@ -739,7 +772,9 @@ def run_b200(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps of the resident-input leg (every k of c5) and launches of the extraction leg; "
+                         "the host-buffer leg runs --e2e-steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="c4", choices=sorted(WORKLOADS))
@@ -751,6 +786,8 @@ def main():
     ap.add_argument("--cpu-large-sample", type=int, default=0,
                     help="--impl reference: bases per step (e.g. 100000000: a table that no longer fits the CPU caches)")
     ap.add_argument("--no-extract", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the timed legs returned in their last step as DIR/<name>.npy (float64)")
     ap.add_argument("--planes", action="store_true",
                     help="reads workload, N = 1: evaluate the WHERE clause with the plane test (DNAGPU_WHERE_FLAG_PLANES)")
     ap.add_argument("--chunks", type=int, default=4, help="--exchange fused: digit sub-ranges the exchange is pipelined in")
