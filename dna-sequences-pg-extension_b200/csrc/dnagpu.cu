@@ -325,9 +325,11 @@ extern "C" int dnagpu_create(dnagpu_ctx **out, int device)
         }
         cudaFuncSetAttribute(k_sort_scatter<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SortSmem));
         cudaFuncSetAttribute(k_sort_scatter<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SortSmem));
-        const int bsmem = kBucketSlots * 12;
+        const int bsmem = kBucketSlots * 12, bsmem64 = kBucketSlots * 16;
         cudaFuncSetAttribute(k_count_buckets<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bsmem);
         cudaFuncSetAttribute(k_count_buckets<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bsmem);
+        cudaFuncSetAttribute(k_count_buckets<false, unsigned long long>, cudaFuncAttributeMaxDynamicSharedMemorySize, bsmem64);
+        cudaFuncSetAttribute(k_count_buckets<true, unsigned long long>, cudaFuncAttributeMaxDynamicSharedMemorySize, bsmem64);
     }
     CU(nullptr, cudaGetLastError());
     *out = ctx;
@@ -1615,6 +1617,17 @@ static int part_level1(dnagpu_ctx *ctx, Scratch &sc, const CountInput &in, int k
     return DNAGPU_OK;
 }
 
+/* k_count_buckets over n keys in all: one key can occur n times, so past 2^32 - 1 keys the per-slot extras
+ * counter is 64-bit (like count_dense_any's counters); every smaller call runs the 32-bit kernel */
+template <bool EMIT, class... A>
+static void launch_count_buckets(dnagpu_ctx *ctx, uint64_t n, unsigned grid, A... a)
+{
+    if (n < 0xffffffffull)
+        k_count_buckets<EMIT, uint32_t><<<grid, kThreads, kBucketSlots * 12, ctx->stream>>>(a...);
+    else
+        k_count_buckets<EMIT, unsigned long long><<<grid, kThreads, kBucketSlots * 16, ctx->stream>>>(a...);
+}
+
 /* Level 2 (inside every parent; parents with equal parent % n_groups merge into the same children)
  * and the shared-memory count of every bucket.  Leaves distinct / unique in the device counters. */
 static int part_finish_impl(dnagpu_ctx *ctx, Scratch &sc, const uint64_t *keys, uint64_t n, const uint64_t *parent_off,
@@ -1698,7 +1711,6 @@ static int part_finish_impl(dnagpu_ctx *ctx, Scratch &sc, const uint64_t *keys, 
         k_table_init<<<(unsigned)std::min<uint64_t>(grid_for(spill_cap, kThreads), (uint64_t)ctx->sm_count * 8),
                        kThreads, 0, ctx->stream>>>(spill, spill_cap);
     }));
-    const int bsmem = kBucketSlots * 12;
     const unsigned cgrid = (unsigned)std::min<uint64_t>(n_buckets, (uint64_t)ctx->sm_count * (16384 / kBucketSlots));
     /* the aggregates: bin / place / compare for every bucket that fits, the table kernel for the rest */
     static const bool use_bins = !tune_env("DNAGPU_NO_BINS");
@@ -1711,14 +1723,14 @@ static int part_finish_impl(dnagpu_ctx *ctx, Scratch &sc, const uint64_t *keys, 
                                                                      ctx->d_ctr, passed, ctx->d_ctr + C_PASSED);
         }));
         TRY(launch(ctx, "count_buckets_passed", [&] {
-            k_count_buckets<false><<<cgrid, kThreads, bsmem, ctx->stream>>>(bucket_keys, bucket_off, bucket_end, n_buckets,
-                                                                           spill, spill_cap, ctx->d_ctr, nullptr, nullptr,
-                                                                           passed, ctx->d_ctr + C_PASSED);
+            launch_count_buckets<false>(ctx, n, cgrid, bucket_keys, bucket_off, bucket_end, n_buckets, spill, spill_cap,
+                                        ctx->d_ctr, (uint64_t *)nullptr, (uint64_t *)nullptr, (const uint32_t *)passed,
+                                        (const unsigned long long *)ctx->d_ctr + C_PASSED);
         }));
     } else {
         TRY(launch(ctx, "count_buckets", [&] {
-            k_count_buckets<false><<<cgrid, kThreads, bsmem, ctx->stream>>>(bucket_keys, bucket_off, bucket_end, n_buckets,
-                                                                           spill, spill_cap, ctx->d_ctr, nullptr, nullptr);
+            launch_count_buckets<false>(ctx, n, cgrid, bucket_keys, bucket_off, bucket_end, n_buckets, spill, spill_cap,
+                                        ctx->d_ctr, (uint64_t *)nullptr, (uint64_t *)nullptr);
         }));
     }
     TRY(fetch_counters(ctx));
@@ -1748,9 +1760,8 @@ static int part_finish_impl(dnagpu_ctx *ctx, Scratch &sc, const uint64_t *keys, 
         if (keyed) {
             CU(ctx, cudaMemsetAsync(ctx->d_ctr + C_CURSOR, 0, 8, ctx->stream));
             TRY(launch(ctx, "count_buckets_emit", [&] {
-                k_count_buckets<true><<<cgrid, kThreads, bsmem, ctx->stream>>>(
-                    bucket_keys, bucket_off, bucket_end, n_buckets, spill, spill_cap, ctx->d_ctr, (*table)->d_kmers,
-                    (*table)->d_counts);
+                launch_count_buckets<true>(ctx, n, cgrid, bucket_keys, bucket_off, bucket_end, n_buckets, spill, spill_cap,
+                                           ctx->d_ctr, (*table)->d_kmers, (*table)->d_counts);
             }));
             TRY(launch(ctx, "table_compact", [&] { /* rows that spilled, appended after the bucket rows */
                 k_table_compact<<<(unsigned)std::min<uint64_t>(grid_for(spill_cap, kThreads), (uint64_t)ctx->sm_count * 8),
@@ -1939,10 +1950,10 @@ static int count_kmers_pipelined(dnagpu_ctx *ctx, const uint64_t *words, uint64_
     if (tune_env("DNAGPU_EXACT_LEVEL1") || pick_method(nullptr, k, rows) != DNAGPU_COUNT_PARTITION) return DNAGPU_OK;
     CU(ctx, cudaSetDevice(ctx->device));
     if (!ctx->copy_stream) CU(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-    Scratch sc(ctx);
+    Scratch words_sc(ctx), sc(ctx); /* the words outlive the optimistic pass's scratch (see the redo below) */
     uint64_t *d_words;
     const uint64_t alloc_words = (n_words + 3) & ~1ull;
-    TRY(sc.get((void **)&d_words, alloc_words * 8));
+    TRY(words_sc.get((void **)&d_words, alloc_words * 8));
     CU(ctx, cudaMemsetAsync(d_words + n_words, 0, (alloc_words - n_words) * 8, ctx->stream));
     int b1, b2;
     plan_bits(rows, 1, &b1, &b2);
@@ -1981,6 +1992,10 @@ static int count_kmers_pipelined(dnagpu_ctx *ctx, const uint64_t *words, uint64_
             dnagpu_table_free(*table);
             *table = nullptr;
         }
+        /* the regions and buckets of the optimistic pass go back to the pool before the exact pass allocates its
+         * own, so the redo needs no more device memory than an exact count of the resident words */
+        for (void *p : sc.ptrs) dfree(ctx, p);
+        sc.ptrs.clear();
         dnagpu_seq *seq = nullptr;
         TRY(dnagpu_seq_wrap(ctx, d_words, n_bases, alloc_words, &seq));
         rc = dnagpu_count(ctx, seq, k, nullptr, nullptr, stats, table);

@@ -792,7 +792,8 @@ struct BucketTally {
 
 /* distinct / unique are accounted at insert time: a claim is a new distinct AND unique key; the
  * first extra occurrence (the add returns 0) takes the key out of the unique set.  No scan. */
-__device__ __forceinline__ void bucket_insert(unsigned long long *tk, uint32_t *tc, uint64_t x, bool spill_ok,
+template <class CT>
+__device__ __forceinline__ void bucket_insert(unsigned long long *tk, CT *tc, uint64_t x, bool spill_ok,
                                               Slot *__restrict__ spill, uint64_t spill_cap, BucketTally &bt,
                                               Tally &ty, unsigned long long *ctr)
 {
@@ -806,7 +807,7 @@ __device__ __forceinline__ void bucket_insert(unsigned long long *tk, uint32_t *
             return;
         }
         if (old == x) {
-            bt.unique -= (atomicAdd(&tc[sl], 1u) == 0);
+            bt.unique -= (atomicAdd(&tc[sl], (CT)1) == 0);
             return;
         }
         sl = (sl + 1) & (kBucketSlots - 1);
@@ -817,7 +818,9 @@ __device__ __forceinline__ void bucket_insert(unsigned long long *tk, uint32_t *
     }
 }
 
-template <bool EMIT>
+/* CT, the per-slot count of extra occurrences: uint32_t unless the call has 2^32 - 1 or more keys, where one key
+ * can occur 2^32 + 1 times and a 32-bit count would wrap (unsigned long long, 16 bytes per slot) */
+template <bool EMIT, class CT = uint32_t>
 __global__ void __launch_bounds__(kThreads) k_count_buckets(const uint64_t *__restrict__ keys,
                                                             const uint64_t *__restrict__ bucket_off,
                                                             const uint64_t *__restrict__ bucket_end,
@@ -833,7 +836,7 @@ __global__ void __launch_bounds__(kThreads) k_count_buckets(const uint64_t *__re
     if (list) n_buckets = *list_n;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     unsigned long long *tk = reinterpret_cast<unsigned long long *>(smem_raw);                /* keys   */
-    uint32_t *tc = reinterpret_cast<uint32_t *>(smem_raw + sizeof(uint64_t) * kBucketSlots); /* extras */
+    CT *tc = reinterpret_cast<CT *>(smem_raw + sizeof(uint64_t) * kBucketSlots); /* extras */
     __shared__ unsigned long long row_base;
     Tally ty = {0, 0, 0, 0}; /* spilled keys account themselves through hash_insert */
     BucketTally bt = {0, 0};
@@ -865,14 +868,14 @@ __global__ void __launch_bounds__(kThreads) k_count_buckets(const uint64_t *__re
             nbeg = bucket_off[id];
             nend = bucket_end[id];
         }
-        { /* 48 KB of 16-byte stores */
+        { /* 48 (64) KB of 16-byte stores */
             ulonglong2 *k2 = reinterpret_cast<ulonglong2 *>(tk);
             uint4 *c4 = reinterpret_cast<uint4 *>(tc);
 #pragma unroll
             for (int i = 0; i < kBucketSlots / 2 / kThreads; ++i)
                 k2[i * kThreads + threadIdx.x] = make_ulonglong2(kEmpty, kEmpty);
 #pragma unroll
-            for (int i = 0; i < kBucketSlots / 4 / kThreads; ++i)
+            for (int i = 0; i < kBucketSlots * (int)sizeof(CT) / 16 / kThreads; ++i)
                 c4[i * kThreads + threadIdx.x] = make_uint4(0, 0, 0, 0);
         }
         CT_MARK(c1);
@@ -902,7 +905,7 @@ __global__ void __launch_bounds__(kThreads) k_count_buckets(const uint64_t *__re
                     bt.distinct++;
                     bt.unique++;
                 } else if (old[u] == pre[u]) {
-                    bt.unique -= (atomicAdd(&tc[sl[u]], 1u) == 0);
+                    bt.unique -= (atomicAdd(&tc[sl[u]], (CT)1) == 0);
                 } else {
                     pending |= 1u << u;
                 }
@@ -930,7 +933,7 @@ __global__ void __launch_bounds__(kThreads) k_count_buckets(const uint64_t *__re
                         bt.unique++;
                         pending &= pending - 1;
                     } else if (o == key) {
-                        bt.unique -= (atomicAdd(&tc[slot], 1u) == 0);
+                        bt.unique -= (atomicAdd(&tc[slot], (CT)1) == 0);
                         pending &= pending - 1;
                     } else if (++probes == kBucketSlots) { /* table full of other keys: count it in HBM */
                         if (!EMIT) hash_insert(spill, spill_cap, key, ty, ctr);
