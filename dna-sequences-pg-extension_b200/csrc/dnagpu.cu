@@ -98,14 +98,6 @@ struct dnagpu_index {
 
 static thread_local char g_err[512] = "";
 
-/* A/B switches of the kernel experiments (profiles/README.md): compiled in only with -DDNAGPU_TUNING
- * (tools/try_alt_lib.sh); the product library reads no environment variables. */
-#ifdef DNAGPU_TUNING
-static inline const char *tune_env(const char *name) { return getenv(name); }
-#else
-static inline const char *tune_env(const char *) { return nullptr; }
-#endif
-
 static int fail(dnagpu_ctx *ctx, int code, const char *fmt, ...)
 {
     char buf[512];
@@ -295,24 +287,18 @@ extern "C" int dnagpu_create(dnagpu_ctx **out, int device)
     {
         const int psmem = kTileKeys * (int)sizeof(uint64_t) + (int)sizeof(ScatterSmem);
 #define PSMEM_ATTR(kern) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, psmem)
-        PSMEM_ATTR((k_part_scatter_seq<kSingle, false>));
-        PSMEM_ATTR((k_part_scatter_seq<kSingle, true>));
-        PSMEM_ATTR((k_part_scatter_seq<kFixed, false>));
-        PSMEM_ATTR((k_part_scatter_seq<kFixed, true>));
-        PSMEM_ATTR((k_part_scatter_seq<kRagged, false>));
-        PSMEM_ATTR((k_part_scatter_seq<kRagged, true>));
         PSMEM_ATTR(k_part_scatter_keys<false>);
         {
             const int psmem32 = 32 * kScatThreads * (int)sizeof(uint64_t) + (int)sizeof(ScatterSmem);
 #define PSMEM32_ATTR(kern) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, psmem32)
             PSMEM32_ATTR((k_part_scatter_keys<false, kBigPerKeys, kBigThreadsKeys>));
             PSMEM32_ATTR((k_part_scatter_keys<true, kBigPerKeys, kBigThreadsKeys>));
-            PSMEM32_ATTR((k_part_scatter_seq<kSingle, false, kBigPer, kBigThreads>));
-            PSMEM32_ATTR((k_part_scatter_seq<kSingle, true, kBigPer, kBigThreads>));
-            PSMEM32_ATTR((k_part_scatter_seq<kFixed, false, kBigPer, kBigThreads>));
-            PSMEM32_ATTR((k_part_scatter_seq<kFixed, true, kBigPer, kBigThreads>));
-            PSMEM32_ATTR((k_part_scatter_seq<kRagged, false, kBigPer, kBigThreads>));
-            PSMEM32_ATTR((k_part_scatter_seq<kRagged, true, kBigPer, kBigThreads>));
+            PSMEM32_ATTR((k_part_scatter_seq<kSingle, false>));
+            PSMEM32_ATTR((k_part_scatter_seq<kSingle, true>));
+            PSMEM32_ATTR((k_part_scatter_seq<kFixed, false>));
+            PSMEM32_ATTR((k_part_scatter_seq<kFixed, true>));
+            PSMEM32_ATTR((k_part_scatter_seq<kRagged, false>));
+            PSMEM32_ATTR((k_part_scatter_seq<kRagged, true>));
 #undef PSMEM32_ATTR
         }
         PSMEM_ATTR(k_part_scatter_keys<true>);
@@ -1044,7 +1030,7 @@ extern "C" int dnagpu_extract(dnagpu_ctx *ctx, const dnagpu_seq *seq, int k, uin
         return fail(ctx, DNAGPU_ECAPACITY, "generate_kmers needs room for %llu rows",
                     (unsigned long long)v.n_rows);
     if ((uintptr_t)d_out & 15) return fail(ctx, DNAGPU_EARG, "d_out must be 16-byte aligned");
-    if (((uintptr_t)d_out & 31) == 0 && !tune_env("DNAGPU_EXTRACT_PAIRS_ONLY")) { /* 256-bit stores */
+    if (((uintptr_t)d_out & 31) == 0) { /* 256-bit stores */
         const unsigned grid = grid_for((v.n_rows + 3) / 4, (uint64_t)kThreads * kQuadsPerThread);
         DISPATCH_LAYOUT(seq->layout, TRY(launch(ctx, "extract", [&] {
             k_extract4<LY><<<grid, kThreads, 0, ctx->stream>>>(v, kmer_mask(k), d_out);
@@ -1379,6 +1365,12 @@ static int count_dense_t(dnagpu_ctx *ctx, const CountInput &in, int k, dnagpu_st
     return DNAGPU_OK;
 }
 
+static int count_dense_any(dnagpu_ctx *ctx, const CountInput &in, int k, dnagpu_stats *stats, dnagpu_table **table)
+{
+    return in.n < 0xffffffffull ? count_dense_t<uint32_t>(ctx, in, k, stats, table)
+                                : count_dense_t<unsigned long long>(ctx, in, k, stats, table);
+}
+
 static int count_hash(dnagpu_ctx *ctx, const CountInput &in, int k, const dnagpu_count_opts *opts,
                       uint64_t n_keys_bound, dnagpu_stats *stats, dnagpu_table **table)
 {
@@ -1446,19 +1438,6 @@ static int count_hash(dnagpu_ctx *ctx, const CountInput &in, int k, const dnagpu
     return DNAGPU_OK;
 }
 
-/* scatter tile: 16384 keys (one CTA per SM) when the fan-out makes 8192-key runs too short */
-static inline bool scatter_tile32(uint32_t fan, int level = 0)
-{
-    if (const char *e = tune_env("DNAGPU_SCATTER_TILE")) return atoi(e) == 16384;
-    if (level == 1)
-        if (const char *e = tune_env("DNAGPU_SCATTER_TILE_L1")) return atoi(e) == 16384;
-    if (level == 2)
-        if (const char *e = tune_env("DNAGPU_SCATTER_TILE_L2")) return atoi(e) == 16384;
-    /* measured: from packed input (level 1) 16384-key tiles win at every fan-out (256: 15 %, 1024: 12 %, 2048: 2x);
-     * from a key list they win 13 % at 2048, 1 % at 1024 and lose 10 % at 256 */
-    return level == 1 || fan >= 1024;
-}
-
 /* exclusive scan of n u64 (out has n + 1 entries); multi-CTA above 16 K entries */
 static int scan_any(dnagpu_ctx *ctx, Scratch &sc, const uint64_t *in, uint64_t n, uint64_t *out)
 {
@@ -1483,8 +1462,6 @@ static int ceil_log2(uint64_t x)
 /* number of hash bits so that a bucket averages at most half the slots of the shared-memory table */
 static int bucket_bits(uint64_t n)
 {
-    if (const char *e = tune_env("DNAGPU_BUCKET_BITS")) /* profiling aid: force the fan-out */
-        if (atoi(e) >= 1 && atoi(e) <= 22) return atoi(e);
     return std::max(1, std::min(22, ceil_log2((n + kBucketSlots / 2 - 1) / (kBucketSlots / 2)))); /* mean <= slots / 2 */
 }
 
@@ -1519,10 +1496,9 @@ static void plan_bits(uint64_t n, uint32_t n_parts, int *b1, int *b2)
 {
     const int b = bucket_bits(n);
     if (n_parts <= 1) {
+        /* the odd bit goes to level 1: level 2 moves twice the bytes per key and gains more from the longer runs of
+         * the smaller fan-out (measured: 50.8 -> 49.9 ms) */
         *b1 = b <= 11 ? b : (b + 1) / 2;
-        if (const char *e = tune_env("DNAGPU_L1_BITS")) /* profiling aid: how the bits split over the two levels */
-            if (atoi(e) >= 1 && atoi(e) <= 11 && b - atoi(e) <= 11) *b1 = atoi(e); /* the odd bit goes to level 1: level 2 moves twice the bytes per key and
-                                          * gains more from the longer runs of the smaller fan-out (measured: 50.8 -> 49.9 ms) */
         *b2 = std::max(0, std::min(11, b - *b1));
         return;
     }
@@ -1532,45 +1508,107 @@ static void plan_bits(uint64_t n, uint32_t n_parts, int *b1, int *b2)
     *b2 = std::max(1, std::min(11, b - *b1));
 }
 
+/* ---- partition level 1: the launches shared by the local count and the multi-GPU exchange ---------------- */
+/* The whole of a key list as the one parent partition the key kernels walk: its range {0, n} on the device.
+ * Synchronises: h_ctr is pinned staging shared with the counters. */
+static int root_range(dnagpu_ctx *ctx, Scratch &sc, uint64_t n, uint64_t **root)
+{
+    TRY(sc.get((void **)root, 2 * 8));
+    ctx->h_ctr[0] = 0;
+    ctx->h_ctr[1] = n;
+    CU(ctx, cudaMemcpyAsync(*root, ctx->h_ctr, 16, cudaMemcpyHostToDevice, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    return DNAGPU_OK;
+}
+
+/* keys per digit of level 1 (1 << b1 digits) into hist (zeroed by the caller), from packed input (the WHERE clause
+ * fused) or from a key list whose root_range is `root` */
+static int l1_hist(dnagpu_ctx *ctx, Scratch &sc, const CountInput &in, int k, int b1, const uint64_t *root,
+                   unsigned long long *hist)
+{
+    const uint32_t P1 = 1u << b1;
+    const int shift1 = 64 - b1;
+    if (in.d_keys) {
+        uint64_t *tiles;
+        TRY(part_tiles(ctx, sc, root, root + 1, 1, kSuperTile, &tiles));
+        return launch(ctx, "part_hist", [&] {
+            k_part_hist_keys<<<grid_for(in.n, kSuperTile), kThreads, 0, ctx->stream>>>(in.d_keys, root, root + 1, tiles, 1, 1,
+                                                                                       shift1, P1, hist);
+        });
+    }
+    const uint64_t mask = kmer_mask(k);
+    const unsigned grid = (unsigned)std::min<uint64_t>(grid_for(in.v.n_items, kThreads), (uint64_t)ctx->sm_count * 8);
+    DISPATCH_LAYOUT(in.seq->layout, TRY(launch(ctx, "part_hist", [&] {
+        if (in.filtered)
+            k_part_hist_seq<LY, true><<<grid, kThreads, 0, ctx->stream>>>(in.v, in.p, mask, shift1, P1, hist);
+        else
+            k_part_hist_seq<LY, false><<<grid, kThreads, 0, ctx->stream>>>(in.v, in.p, mask, shift1, P1, hist);
+    })));
+    return DNAGPU_OK;
+}
+
+/* Level-1 scatter of packed input: digit d's keys go to out[child_off[d] + child_cur[d] ...]; with cap != 0
+ * (optimistic regions) a run that finds its region full is dropped and raises C_L1OVF.  16384-key tiles,
+ * kBigThreads x kBigPer: measured from packed input they win over 8192-key tiles at every fan-out (256: 15 %,
+ * 1024: 12 %, 2048: 2x).  out == NULL: child_off holds destination addresses / 8 (peer_dest), the stores go to
+ * peer memory. */
+static int l1_scatter_seq(dnagpu_ctx *ctx, int layout, const SeqView &v, const Pred &p, bool filtered, int k, int b1,
+                          const uint64_t *child_off, unsigned long long *child_cur, uint64_t *out, uint64_t cap)
+{
+    const uint32_t P1 = 1u << b1;
+    const int shift1 = 64 - b1;
+    const uint64_t mask = kmer_mask(k);
+    const int psmem = kBigPer * kBigThreads * (int)sizeof(uint64_t) + (int)sizeof(ScatterSmem);
+    const unsigned grid = grid_for(v.n_items, kBigPer * kBigThreads / 32); /* packed items (32 starts) per tile */
+    DISPATCH_LAYOUT(layout, TRY(launch(ctx, out ? "part_scatter" : "part_scatter_peer", [&] {
+        if (filtered)
+            k_part_scatter_seq<LY, true><<<grid, kBigThreads, psmem, ctx->stream>>>(v, p, mask, shift1, P1, child_off,
+                                                                                   child_cur, out, ctx->d_ctr, cap);
+        else
+            k_part_scatter_seq<LY, false><<<grid, kBigThreads, psmem, ctx->stream>>>(v, p, mask, shift1, P1, child_off,
+                                                                                    child_cur, out, ctx->d_ctr, cap);
+    })));
+    return DNAGPU_OK;
+}
+
+/* The same from a key list whose root_range is `root`; its 'G' x 32 keys are counted aside.  tile32: 16384-key tiles
+ * (kBigThreadsKeys x kBigPerKeys) instead of 8192: measured from a key list they win 13 % at a fan-out of 2048, 1 % at
+ * 1024 and lose 10 % at 256. */
+static int l1_scatter_keys(dnagpu_ctx *ctx, Scratch &sc, const uint64_t *keys, uint64_t n, const uint64_t *root, bool tile32,
+                           int b1, const uint64_t *child_off, unsigned long long *child_cur, uint64_t *out, uint64_t cap)
+{
+    const uint32_t P1 = 1u << b1;
+    const int shift1 = 64 - b1;
+    const uint64_t tile = tile32 ? 2 * kTileKeys : kTileKeys;
+    uint64_t *tiles;
+    TRY(part_tiles(ctx, sc, root, root + 1, 1, tile, &tiles));
+    const int psmem = (int)tile * (int)sizeof(uint64_t) + (int)sizeof(ScatterSmem);
+    return launch(ctx, out ? "part_scatter" : "part_scatter_peer", [&] {
+        if (tile32)
+            k_part_scatter_keys<true, kBigPerKeys, kBigThreadsKeys><<<grid_for(n, tile), kBigThreadsKeys, psmem, ctx->stream>>>(
+                keys, root, root + 1, tiles, 1, 1, shift1, P1, child_off, child_cur, out, ctx->d_ctr, cap, C_L1OVF);
+        else
+            k_part_scatter_keys<true><<<grid_for(n, tile), kScatThreads, psmem, ctx->stream>>>(
+                keys, root, root + 1, tiles, 1, 1, shift1, P1, child_off, child_cur, out, ctx->d_ctr, cap, C_L1OVF);
+    });
+}
+
 /* Level 1: histogram, offsets (off1: device, P1 + 1 entries) and scatter into `out` (>= n + 2 keys).
  * The device counters C_TOTAL / C_SIDE receive the rows kept by the WHERE clause / the 'G' x 32 rows. */
 static int part_level1(dnagpu_ctx *ctx, Scratch &sc, const CountInput &in, int k, int b1, uint64_t **keys_io,
                        uint64_t cap, uint64_t **off1_out, uint64_t *n_out)
 {
-    const uint64_t mask = kmer_mask(k);
-    const int psmem = kTileKeys * (int)sizeof(uint64_t) + (int)sizeof(ScatterSmem);
     const uint32_t P1 = 1u << b1;
-    const int shift1 = 64 - b1;
     uint64_t n = in.n;
     unsigned long long *hist1, *cur1;
-    uint64_t *off1, *root_off;
+    uint64_t *off1, *root = nullptr;
     TRY(sc.get((void **)&hist1, (uint64_t)P1 * 8));
     TRY(sc.get((void **)&cur1, (uint64_t)P1 * 8));
     TRY(sc.get((void **)&off1, ((uint64_t)P1 + 1) * 8));
-    TRY(sc.get((void **)&root_off, 2 * 8));
     CU(ctx, cudaMemsetAsync(hist1, 0, (uint64_t)P1 * 8, ctx->stream));
     CU(ctx, cudaMemsetAsync(cur1, 0, (uint64_t)P1 * 8, ctx->stream));
-    uint64_t *root_tiles_hist = nullptr, *root_tiles_scat = nullptr;
-    if (in.d_keys) {
-        ctx->h_ctr[0] = 0;
-        ctx->h_ctr[1] = n;
-        CU(ctx, cudaMemcpyAsync(root_off, ctx->h_ctr, 16, cudaMemcpyHostToDevice, ctx->stream));
-        CU(ctx, cudaStreamSynchronize(ctx->stream)); /* h_ctr is reused below */
-        TRY(part_tiles(ctx, sc, root_off, root_off + 1, 1, kSuperTile, &root_tiles_hist));
-        TRY(part_tiles(ctx, sc, root_off, root_off + 1, 1, kTileKeys, &root_tiles_scat));
-        TRY(launch(ctx, "part_hist", [&] {
-            k_part_hist_keys<<<grid_for(n, kSuperTile), kThreads, 0, ctx->stream>>>(
-                in.d_keys, root_off, root_off + 1, root_tiles_hist, 1, 1, shift1, P1, hist1);
-        }));
-    } else {
-        const unsigned hgrid = (unsigned)std::min<uint64_t>(grid_for(in.v.n_items, kThreads), (uint64_t)ctx->sm_count * 8);
-        DISPATCH_LAYOUT(in.seq->layout, TRY(launch(ctx, "part_hist", [&] {
-            if (in.filtered)
-                k_part_hist_seq<LY, true><<<hgrid, kThreads, 0, ctx->stream>>>(in.v, in.p, mask, shift1, P1, hist1);
-            else
-                k_part_hist_seq<LY, false><<<hgrid, kThreads, 0, ctx->stream>>>(in.v, in.p, mask, shift1, P1, hist1);
-        })));
-    }
+    if (in.d_keys) TRY(root_range(ctx, sc, n, &root));
+    TRY(l1_hist(ctx, sc, in, k, b1, root, hist1));
     TRY(scan_any(ctx, sc, (const uint64_t *)hist1, P1, off1));
     uint64_t *out = *keys_io;
     if (in.filtered || out) /* the WHERE clause decides how many keys there are; a caller's buffer must fit them */
@@ -1582,36 +1620,12 @@ static int part_level1(dnagpu_ctx *ctx, Scratch &sc, const CountInput &in, int k
         *n_out = n;
         return fail(ctx, DNAGPU_ECAPACITY, "partition needs room for %llu keys (+2 pad)", (unsigned long long)n);
     }
-    if (in.d_keys) {
-        TRY(launch(ctx, "part_scatter", [&] {
-            k_part_scatter_keys<true><<<grid_for(in.n, kTileKeys), kScatThreads, psmem, ctx->stream>>>(
-                in.d_keys, root_off, root_off + 1, root_tiles_scat, 1, 1, shift1, P1, off1, cur1, out, ctx->d_ctr);
-        }));
-    } else {
-        const bool per32 = scatter_tile32(P1, in.d_keys ? 0 : 1);
-        if (per32) {
-            const int psmem32 = 32 * kScatThreads * (int)sizeof(uint64_t) + (int)sizeof(ScatterSmem);
-            const unsigned grid = grid_for(in.v.n_items, kScatThreads);
-            DISPATCH_LAYOUT(in.seq->layout, TRY(launch(ctx, "part_scatter", [&] {
-                if (in.filtered)
-                    k_part_scatter_seq<LY, true, kBigPer, kBigThreads><<<grid, kBigThreads, psmem32, ctx->stream>>>(
-                        in.v, in.p, mask, shift1, P1, off1, cur1, out, ctx->d_ctr, 0);
-                else
-                    k_part_scatter_seq<LY, false, kBigPer, kBigThreads><<<grid, kBigThreads, psmem32, ctx->stream>>>(
-                        in.v, in.p, mask, shift1, P1, off1, cur1, out, ctx->d_ctr, 0);
-            })));
-        } else {
-            const unsigned grid = grid_for(in.v.n_items, kScatThreads / 2);
-            DISPATCH_LAYOUT(in.seq->layout, TRY(launch(ctx, "part_scatter", [&] {
-                if (in.filtered)
-                    k_part_scatter_seq<LY, true><<<grid, kScatThreads, psmem, ctx->stream>>>(
-                        in.v, in.p, mask, shift1, P1, off1, cur1, out, ctx->d_ctr, 0);
-                else
-                    k_part_scatter_seq<LY, false><<<grid, kScatThreads, psmem, ctx->stream>>>(
-                        in.v, in.p, mask, shift1, P1, off1, cur1, out, ctx->d_ctr, 0);
-            })));
-        }
-    }
+    /* 8192-key tiles from a key list: this exact form counts lists under 2^24 keys, DNAGPU_COUNT_FLAG_EXACT queries and
+     * the redo of an optimistic level 1 that found a region full */
+    if (in.d_keys)
+        TRY(l1_scatter_keys(ctx, sc, in.d_keys, in.n, root, false, b1, off1, cur1, out, 0));
+    else
+        TRY(l1_scatter_seq(ctx, in.seq->layout, in.v, in.p, in.filtered, k, b1, off1, cur1, out, 0));
     *off1_out = off1;
     *n_out = n;
     return DNAGPU_OK;
@@ -1669,7 +1683,7 @@ static int part_finish_impl(dnagpu_ctx *ctx, Scratch &sc, const uint64_t *keys, 
         }
         /* measured on the headline workload: at a fan-out of 2048 a (tile, digit) run of an 8192-key tile
          * is only 4 keys; 16384-key tiles (one CTA per SM) win 13 % there, are even at 1024 and lose 10 % at 256 */
-        const bool per32 = scatter_tile32(P2, 2);
+        const bool per32 = P2 >= 1024;
         TRY(part_tiles(ctx, sc, parent_off, parent_end, n_parents, per32 ? 2 * kTileKeys : kTileKeys, &tiles_scat, &tparent_scat,
                        (uint64_t)grid_for(n, per32 ? 2 * kTileKeys : kTileKeys) + n_parents));
         if (!optimistic2) {
@@ -1713,41 +1727,23 @@ static int part_finish_impl(dnagpu_ctx *ctx, Scratch &sc, const uint64_t *keys, 
     }));
     const unsigned cgrid = (unsigned)std::min<uint64_t>(n_buckets, (uint64_t)ctx->sm_count * (16384 / kBucketSlots));
     /* the aggregates: bin / place / compare for every bucket that fits, the table kernel for the rest */
-    static const bool use_bins = !tune_env("DNAGPU_NO_BINS");
-    if (use_bins) {
-        uint32_t *passed;
-        TRY(sc.get((void **)&passed, n_buckets * 4 + 16));
-        const unsigned bgrid = (unsigned)std::min<uint64_t>(n_buckets, (uint64_t)ctx->sm_count * ctx->bins_ctas_per_sm);
-        TRY(launch(ctx, "count_buckets", [&] {
-            k_count_buckets_bins<<<bgrid, kThreads, 0, ctx->stream>>>(bucket_keys, bucket_off, bucket_end, n_buckets,
-                                                                     ctx->d_ctr, passed, ctx->d_ctr + C_PASSED);
-        }));
-        TRY(launch(ctx, "count_buckets_passed", [&] {
-            launch_count_buckets<false>(ctx, n, cgrid, bucket_keys, bucket_off, bucket_end, n_buckets, spill, spill_cap,
-                                        ctx->d_ctr, (uint64_t *)nullptr, (uint64_t *)nullptr, (const uint32_t *)passed,
-                                        (const unsigned long long *)ctx->d_ctr + C_PASSED);
-        }));
-    } else {
-        TRY(launch(ctx, "count_buckets", [&] {
-            launch_count_buckets<false>(ctx, n, cgrid, bucket_keys, bucket_off, bucket_end, n_buckets, spill, spill_cap,
-                                        ctx->d_ctr, (uint64_t *)nullptr, (uint64_t *)nullptr);
-        }));
-    }
+    uint32_t *passed;
+    TRY(sc.get((void **)&passed, n_buckets * 4 + 16));
+    const unsigned bgrid = (unsigned)std::min<uint64_t>(n_buckets, (uint64_t)ctx->sm_count * ctx->bins_ctas_per_sm);
+    TRY(launch(ctx, "count_buckets", [&] {
+        k_count_buckets_bins<<<bgrid, kThreads, 0, ctx->stream>>>(bucket_keys, bucket_off, bucket_end, n_buckets,
+                                                                 ctx->d_ctr, passed, ctx->d_ctr + C_PASSED);
+    }));
+    TRY(launch(ctx, "count_buckets_passed", [&] {
+        launch_count_buckets<false>(ctx, n, cgrid, bucket_keys, bucket_off, bucket_end, n_buckets, spill, spill_cap,
+                                    ctx->d_ctr, (uint64_t *)nullptr, (uint64_t *)nullptr, (const uint32_t *)passed,
+                                    (const unsigned long long *)ctx->d_ctr + C_PASSED);
+    }));
     TRY(fetch_counters(ctx));
     if (ctx->h_ctr[C_L2OVF]) { /* some keys were dropped: the caller redoes level 2 exactly */
         *regions_full = true;
         return DNAGPU_OK;
     }
-#ifdef DNAGPU_PHASE_TIMING
-    fprintf(stderr, "count_buckets phases (cycles/bucket, thread 0): init %.0f | sync %.0f | insert %.0f | prefetch+sync %.0f | buckets %llu\n",
-            (double)ctx->h_ctr[110] / ctx->h_ctr[114], (double)ctx->h_ctr[111] / ctx->h_ctr[114],
-            (double)ctx->h_ctr[112] / ctx->h_ctr[114], (double)ctx->h_ctr[113] / ctx->h_ctr[114],
-            (unsigned long long)ctx->h_ctr[114]);
-    fprintf(stderr, "scatter_seq phases (cycles/tile, thread 0): load+rank %.0f | barrier %.0f | plan %.0f | place %.0f+sync | flush %.0f | tiles %llu\n",
-            (double)ctx->h_ctr[100] / ctx->h_ctr[105], (double)ctx->h_ctr[101] / ctx->h_ctr[105],
-            (double)ctx->h_ctr[102] / ctx->h_ctr[105], (double)ctx->h_ctr[103] / ctx->h_ctr[105],
-            (double)ctx->h_ctr[104] / ctx->h_ctr[105], (unsigned long long)ctx->h_ctr[105]);
-#endif
     if (ctx->h_ctr[C_OVERFLOW])
         return fail(ctx, DNAGPU_EINTERNAL, "spill table of %llu slots overflowed", (unsigned long long)spill_cap);
     const uint64_t side = ctx->h_ctr[C_SIDE];
@@ -1785,8 +1781,7 @@ static int part_finish(dnagpu_ctx *ctx, Scratch &sc, const uint64_t *keys, uint6
                        dnagpu_stats *stats, uint64_t total_rows, dnagpu_table **table)
 {
     /* optimistic level 2 where no parents merge (one GPU) and the buckets are full-sized */
-    static const bool allow = !tune_env("DNAGPU_EXACT_L2");
-    const bool optimistic2 = allow && !ctx->force_exact && b2 > 0 && n_groups == n_parents && (n >> (b1 + b2)) >= 512;
+    const bool optimistic2 = !ctx->force_exact && b2 > 0 && n_groups == n_parents && (n >> (b1 + b2)) >= 512;
     bool full = false;
     TRY(part_finish_impl(ctx, sc, keys, n, parent_off, parent_end, n_parents, n_groups, b1, b2, k, stats, total_rows, table,
                          optimistic2, &full));
@@ -1835,40 +1830,16 @@ static int l1_regions_begin(dnagpu_ctx *ctx, Scratch &sc, uint64_t n_rows, int b
 static int l1_regions_scatter(dnagpu_ctx *ctx, const L1Regions &r, int layout, const SeqView &v, int k)
 {
     const Pred none = {~0ull, ~0ull, ~0ull, ~0ull};
-    if (scatter_tile32(r.P1, 1)) {
-        const int psmem = 32 * kScatThreads * (int)sizeof(uint64_t) + (int)sizeof(ScatterSmem);
-        const unsigned grid = grid_for(v.n_items, kScatThreads);
-        DISPATCH_LAYOUT(layout, TRY(launch(ctx, "part_scatter", [&] {
-            k_part_scatter_seq<LY, false, kBigPer, kBigThreads><<<grid, kBigThreads, psmem, ctx->stream>>>(
-                v, none, kmer_mask(k), 64 - r.b1, r.P1, r.beg, r.cur, r.keys, ctx->d_ctr, r.cap);
-        })));
-        return DNAGPU_OK;
-    }
-    const int psmem = kTileKeys * (int)sizeof(uint64_t) + (int)sizeof(ScatterSmem);
-    const unsigned grid = grid_for(v.n_items, kScatThreads / 2);
-    DISPATCH_LAYOUT(layout, TRY(launch(ctx, "part_scatter", [&] {
-        k_part_scatter_seq<LY, false><<<grid, kScatThreads, psmem, ctx->stream>>>(
-            v, none, kmer_mask(k), 64 - r.b1, r.P1, r.beg, r.cur, r.keys, ctx->d_ctr, r.cap);
-    })));
-    return DNAGPU_OK;
+    return l1_scatter_seq(ctx, layout, v, none, false, k, r.b1, r.beg, r.cur, r.keys, r.cap);
 }
 
 /* the same from a key list on the device (the owned k-mers of a multi-GPU count, a stored column): 16384-key tiles,
- * 'G' x 32 keys counted aside, a full region raises C_L1OVF */
+ * 'G' x 32 keys counted aside */
 static int l1_regions_scatter_keys(dnagpu_ctx *ctx, Scratch &sc, const L1Regions &r, const uint64_t *d_keys, uint64_t n)
 {
-    uint64_t *root_off, *tiles;
-    TRY(sc.get((void **)&root_off, 2 * 8));
-    ctx->h_ctr[C_COUNT] = 0;
-    ctx->h_ctr[C_COUNT + 1] = n;
-    CU(ctx, cudaMemcpyAsync(root_off, ctx->h_ctr + C_COUNT, 16, cudaMemcpyHostToDevice, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream)); /* pinned staging shared with the counters */
-    TRY(part_tiles(ctx, sc, root_off, root_off + 1, 1, 2 * kTileKeys, &tiles));
-    const int psmem32 = 32 * kScatThreads * (int)sizeof(uint64_t) + (int)sizeof(ScatterSmem);
-    return launch(ctx, "part_scatter", [&] {
-        k_part_scatter_keys<true, kBigPerKeys, kBigThreadsKeys><<<grid_for(n, 2 * kTileKeys), kBigThreadsKeys, psmem32, ctx->stream>>>(
-            d_keys, root_off, root_off + 1, tiles, 1, 1, 64 - r.b1, r.P1, r.beg, r.cur, r.keys, ctx->d_ctr, r.cap, C_L1OVF);
-    });
+    uint64_t *root;
+    TRY(root_range(ctx, sc, n, &root));
+    return l1_scatter_keys(ctx, sc, d_keys, n, root, true, r.b1, r.beg, r.cur, r.keys, r.cap);
 }
 
 static int l1_regions_end(dnagpu_ctx *ctx, const L1Regions &r)
@@ -1899,8 +1870,7 @@ static int count_partition_exact(dnagpu_ctx *ctx, const CountInput &in, int k, d
 static int count_partition(dnagpu_ctx *ctx, const CountInput &in, int k, dnagpu_stats *stats,
                            dnagpu_table **table)
 {
-    static const bool no_optimistic = tune_env("DNAGPU_EXACT_LEVEL1") != nullptr;
-    if (in.filtered || no_optimistic || ctx->force_exact || (in.d_keys && in.n < (1ull << 24)))
+    if (in.filtered || ctx->force_exact || (in.d_keys && in.n < (1ull << 24)))
         return count_partition_exact(ctx, in, k, stats, table);
     {
         Scratch sc(ctx);
@@ -1922,6 +1892,30 @@ static int count_partition(dnagpu_ctx *ctx, const CountInput &in, int k, dnagpu_
         }
     }
     return count_partition_exact(ctx, in, k, stats, table); /* a region overflowed: heavily repeated input */
+}
+
+/* rc of a count; a failed count leaves no table behind */
+static int free_table_on_error(int rc, dnagpu_table **table)
+{
+    if (rc != DNAGPU_OK && table && *table) {
+        dnagpu_table_free(*table);
+        *table = nullptr;
+    }
+    return rc;
+}
+
+/* the count itself, by the method pick_method chose */
+static int count_by_method(dnagpu_ctx *ctx, const CountInput &in, int k, int method, const dnagpu_count_opts *opts,
+                           uint64_t n_keys_bound, dnagpu_stats *stats, dnagpu_table **table)
+{
+    int rc;
+    if (method == DNAGPU_COUNT_DENSE)
+        rc = count_dense_any(ctx, in, k, stats, table);
+    else if (method == DNAGPU_COUNT_PARTITION)
+        rc = count_partition(ctx, in, k, stats, table);
+    else
+        rc = count_hash(ctx, in, k, opts, n_keys_bound, stats, table);
+    return free_table_on_error(rc, table);
 }
 
 /* one chunk of a pipelined upload: H2D on the copy stream, the compute stream waits for it.  Never returns
@@ -1947,7 +1941,7 @@ static int count_kmers_pipelined(dnagpu_ctx *ctx, const uint64_t *words, uint64_
 {
     *done = false;
     const uint64_t rows = rows_of(n_bases, k), n_words = words_of(n_bases);
-    if (tune_env("DNAGPU_EXACT_LEVEL1") || pick_method(nullptr, k, rows) != DNAGPU_COUNT_PARTITION) return DNAGPU_OK;
+    if (pick_method(nullptr, k, rows) != DNAGPU_COUNT_PARTITION) return DNAGPU_OK;
     CU(ctx, cudaSetDevice(ctx->device));
     if (!ctx->copy_stream) CU(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
     Scratch words_sc(ctx), sc(ctx); /* the words outlive the optimistic pass's scratch (see the redo below) */
@@ -2039,8 +2033,6 @@ static int collect_rows(dnagpu_ctx *ctx, const CountInput &in, int k, uint64_t *
     return read_u64(ctx, (const uint64_t *)(ctx->d_ctr + C_CURSOR), n_match);
 }
 
-static int count_dense_any(dnagpu_ctx *ctx, const CountInput &in, int k, dnagpu_stats *stats, dnagpu_table **table);
-static int count_partition(dnagpu_ctx *ctx, const CountInput &in, int k, dnagpu_stats *stats, dnagpu_table **table);
 static int count_listed(dnagpu_ctx *ctx, const uint64_t *keys, uint64_t n_match, int k, const dnagpu_count_opts *opts,
                         dnagpu_stats *stats, dnagpu_table **table);
 
@@ -2162,25 +2154,7 @@ static int count_listed(dnagpu_ctx *ctx, const uint64_t *keys, uint64_t n_match,
     listed.d_keys = keys;
     listed.n = n_match;
     dnagpu_count_opts o2 = opts ? *opts : dnagpu_count_opts{0, 0, 0.0, 0, 0, 0};
-    const int method = pick_method(&o2, k, n_match);
-    int rc;
-    if (method == DNAGPU_COUNT_DENSE)
-        rc = count_dense_any(ctx, listed, k, stats, table);
-    else if (method == DNAGPU_COUNT_PARTITION)
-        rc = count_partition(ctx, listed, k, stats, table);
-    else
-        rc = count_hash(ctx, listed, k, opts, n_match, stats, table);
-    if (rc != DNAGPU_OK && table && *table) {
-        dnagpu_table_free(*table);
-        *table = nullptr;
-    }
-    return rc;
-}
-
-static int count_dense_any(dnagpu_ctx *ctx, const CountInput &in, int k, dnagpu_stats *stats, dnagpu_table **table)
-{
-    return in.n < 0xffffffffull ? count_dense_t<uint32_t>(ctx, in, k, stats, table)
-                                : count_dense_t<unsigned long long>(ctx, in, k, stats, table);
+    return count_by_method(ctx, listed, k, pick_method(&o2, k, n_match), opts, n_match, stats, table);
 }
 
 static int count_any(dnagpu_ctx *ctx, CountInput &in, int k, const dnagpu_count_opts *opts,
@@ -2194,8 +2168,7 @@ static int count_any(dnagpu_ctx *ctx, CountInput &in, int k, const dnagpu_count_
         if (table) TRY(table_new(ctx, k, 0, table));
         return DNAGPU_OK;
     }
-    int method = pick_method(opts, k, in.n);
-    int rc;
+    const int method = pick_method(opts, k, in.n);
     struct ExactScope { /* the flag holds for this query only */
         dnagpu_ctx *c;
         ~ExactScope() { c->force_exact = false; }
@@ -2224,28 +2197,10 @@ static int count_any(dnagpu_ctx *ctx, CountInput &in, int k, const dnagpu_count_
             return DNAGPU_OK;
         }
         if (n_match <= in.n / 2 || method == DNAGPU_COUNT_PARTITION) return count_listed(ctx, keys, n_match, k, opts, stats, table);
-        if (method == DNAGPU_COUNT_HASH) { /* not selective: fused insert into a table sized by n_match */
-            rc = count_hash(ctx, in, k, opts, n_match, stats, table);
-            if (rc != DNAGPU_OK && table && *table) {
-                dnagpu_table_free(*table);
-                *table = nullptr;
-            }
-            return rc;
-        }
+        if (method == DNAGPU_COUNT_HASH) /* not selective: fused insert into a table sized by n_match */
+            return count_by_method(ctx, in, k, method, opts, n_match, stats, table);
     }
-    if (method == DNAGPU_COUNT_DENSE) {
-        rc = in.n < 0xffffffffull ? count_dense_t<uint32_t>(ctx, in, k, stats, table)
-                                  : count_dense_t<unsigned long long>(ctx, in, k, stats, table);
-    } else if (method == DNAGPU_COUNT_PARTITION) {
-        rc = count_partition(ctx, in, k, stats, table);
-    } else {
-        rc = count_hash(ctx, in, k, opts, in.n, stats, table);
-    }
-    if (rc != DNAGPU_OK && table && *table) {
-        dnagpu_table_free(*table);
-        *table = nullptr;
-    }
-    return rc;
+    return count_by_method(ctx, in, k, method, opts, in.n, stats, table);
 }
 
 extern "C" int dnagpu_collect(dnagpu_ctx *ctx, const dnagpu_seq *seq, int k, const dnagpu_where *filter,
@@ -2432,7 +2387,7 @@ static int count_reads_pipelined(dnagpu_ctx *ctx, const uint64_t *words, uint64_
     *done = false;
     const uint64_t rows_per_read = rows_of(bases_per_read, k), n = n_reads * rows_per_read;
     if (!words || n < (1ull << 24) || stride_words < words_of(bases_per_read) ||
-        pick_method(nullptr, k, n) == DNAGPU_COUNT_DENSE || tune_env("DNAGPU_NO_READS_PIPELINE"))
+        pick_method(nullptr, k, n) == DNAGPU_COUNT_DENSE)
         return DNAGPU_OK;
     CU(ctx, cudaSetDevice(ctx->device));
     Pred p;
@@ -2720,13 +2675,9 @@ extern "C" int dnagpu_shuffle_count(dnagpu_ctx *ctx, const uint64_t *d_keys, con
     CU(ctx, cudaMemcpyAsync(d_off, off.data(), off.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream)); /* `off` is a host temporary */
     TRY(zero_counters(ctx));
-    int rc = part_finish(ctx, sc, d_keys, n, d_off, d_off + 1, n_pieces, n_groups, plan->bits1, plan->bits2, k, stats, n,
-                         table);
-    if (rc != DNAGPU_OK && table && *table) {
-        dnagpu_table_free(*table);
-        *table = nullptr;
-    }
-    return rc;
+    return free_table_on_error(part_finish(ctx, sc, d_keys, n, d_off, d_off + 1, n_pieces, n_groups, plan->bits1, plan->bits2,
+                                           k, stats, n, table),
+                               table);
 }
 
 /* ---- the exchange fused into the scatter kernel: stores straight into peer memory ---------------- */
@@ -2798,30 +2749,49 @@ static int shuffle_input(dnagpu_ctx *ctx, const dnagpu_seq *seq, int k, const dn
     return build_pred(ctx, filter, k, in->n, &in->p, &in->filtered);
 }
 
+/* keys per digit of level 1 (host array of plan->n_digits entries) of a sequence or a key list */
+static int shuffle_hist(dnagpu_ctx *ctx, const CountInput &in, int k, const dnagpu_shuffle_plan *plan, uint64_t *digit_counts)
+{
+    const uint32_t P1 = plan->n_digits;
+    for (uint32_t d = 0; d < P1; ++d) digit_counts[d] = 0;
+    if (in.n == 0) return DNAGPU_OK;
+    Scratch sc(ctx);
+    unsigned long long *hist1;
+    uint64_t *root = nullptr;
+    TRY(sc.get((void **)&hist1, (uint64_t)P1 * 8));
+    CU(ctx, cudaMemsetAsync(hist1, 0, (uint64_t)P1 * 8, ctx->stream));
+    if (in.d_keys) TRY(root_range(ctx, sc, in.n, &root));
+    TRY(l1_hist(ctx, sc, in, k, plan->bits1, root, hist1));
+    CU(ctx, cudaMemcpyAsync(digit_counts, hist1, (uint64_t)P1 * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    return DNAGPU_OK;
+}
+
 extern "C" int dnagpu_shuffle_hist(dnagpu_ctx *ctx, const dnagpu_seq *seq, int k, const dnagpu_where *filter,
                                    const dnagpu_shuffle_plan *plan, uint64_t *digit_counts)
 {
     if (!ctx || !seq || !plan || !digit_counts) return fail(ctx, DNAGPU_EARG, "dnagpu_shuffle_hist: NULL argument");
     CountInput in;
     TRY(shuffle_input(ctx, seq, k, filter, &in));
-    for (uint32_t d = 0; d < plan->n_digits; ++d) digit_counts[d] = 0;
-    if (in.n == 0) return DNAGPU_OK;
-    Scratch sc(ctx);
+    return shuffle_hist(ctx, in, k, plan, digit_counts);
+}
+
+/* The scatter kernels add "index of the run" to a base pointer; with a NULL base and addresses / 8 as indices the
+ * same kernels store to arbitrary (peer) destinations per digit.  -> that index table and a zeroed cursor per digit. */
+static int peer_dest(dnagpu_ctx *ctx, Scratch &sc, const dnagpu_shuffle_plan *plan, const uint64_t *digit_dest,
+                     uint64_t **d_idx, unsigned long long **cur1)
+{
     const uint32_t P1 = plan->n_digits;
-    unsigned long long *hist1;
-    TRY(sc.get((void **)&hist1, (uint64_t)P1 * 8));
-    CU(ctx, cudaMemsetAsync(hist1, 0, (uint64_t)P1 * 8, ctx->stream));
-    const uint64_t mask = kmer_mask(k);
-    const int shift1 = 64 - plan->bits1;
-    const unsigned hgrid = (unsigned)std::min<uint64_t>(grid_for(in.v.n_items, kThreads), (uint64_t)ctx->sm_count * 8);
-    DISPATCH_LAYOUT(seq->layout, TRY(launch(ctx, "part_hist", [&] {
-        if (in.filtered)
-            k_part_hist_seq<LY, true><<<hgrid, kThreads, 0, ctx->stream>>>(in.v, in.p, mask, shift1, P1, hist1);
-        else
-            k_part_hist_seq<LY, false><<<hgrid, kThreads, 0, ctx->stream>>>(in.v, in.p, mask, shift1, P1, hist1);
-    })));
-    CU(ctx, cudaMemcpyAsync(digit_counts, hist1, (uint64_t)P1 * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    std::vector<uint64_t> idx(P1);
+    for (uint32_t d = 0; d < P1; ++d) {
+        if (digit_dest[d] & 7) return fail(ctx, DNAGPU_EARG, "destination of digit %u is not 8-byte aligned", d);
+        idx[d] = digit_dest[d] >> 3;
+    }
+    TRY(sc.get((void **)d_idx, ((uint64_t)P1 + 1) * 8));
+    TRY(sc.get((void **)cur1, (uint64_t)P1 * 8));
+    CU(ctx, cudaMemcpyAsync(*d_idx, idx.data(), (uint64_t)P1 * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CU(ctx, cudaMemsetAsync(*cur1, 0, (uint64_t)P1 * 8, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream)); /* idx is a host temporary */
     return DNAGPU_OK;
 }
 
@@ -2837,36 +2807,11 @@ extern "C" int dnagpu_shuffle_scatter_to(dnagpu_ctx *ctx, const dnagpu_seq *seq,
     if (side_rows) *side_rows = 0;
     if (in.n == 0) return DNAGPU_OK;
     Scratch sc(ctx);
-    const uint32_t P1 = plan->n_digits;
-    /* the kernel adds "index of the run" to a base pointer; with a NULL base and addresses / 8
-     * as indices the same kernel stores to arbitrary (peer) destinations per digit */
-    std::vector<uint64_t> idx(P1);
-    for (uint32_t d = 0; d < P1; ++d) {
-        if (digit_dest[d] & 7) return fail(ctx, DNAGPU_EARG, "destination of digit %u is not 8-byte aligned", d);
-        idx[d] = digit_dest[d] >> 3;
-    }
     uint64_t *d_idx;
     unsigned long long *cur1;
-    TRY(sc.get((void **)&d_idx, ((uint64_t)P1 + 1) * 8));
-    TRY(sc.get((void **)&cur1, (uint64_t)P1 * 8));
-    CU(ctx, cudaMemcpyAsync(d_idx, idx.data(), (uint64_t)P1 * 8, cudaMemcpyHostToDevice, ctx->stream));
-    CU(ctx, cudaMemsetAsync(cur1, 0, (uint64_t)P1 * 8, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream)); /* idx is a host temporary */
+    TRY(peer_dest(ctx, sc, plan, digit_dest, &d_idx, &cur1));
     TRY(zero_counters(ctx));
-    const uint64_t mask = kmer_mask(k);
-    const int shift1 = 64 - plan->bits1;
-    /* 16384-key tiles (one CTA per SM): a (tile, digit) run is twice as long as in the local scatter,
-     * which is what the NVLink stores want */
-    const int psmem = 32 * kScatThreads * (int)sizeof(uint64_t) + (int)sizeof(ScatterSmem);
-    const unsigned grid = grid_for(in.v.n_items, kScatThreads);
-    DISPATCH_LAYOUT(seq->layout, TRY(launch(ctx, "part_scatter_peer", [&] {
-        if (in.filtered)
-            k_part_scatter_seq<LY, true, kBigPer, kBigThreads><<<grid, kBigThreads, psmem, ctx->stream>>>(
-                in.v, in.p, mask, shift1, P1, d_idx, cur1, (uint64_t *)nullptr, ctx->d_ctr, 0);
-        else
-            k_part_scatter_seq<LY, false, kBigPer, kBigThreads><<<grid, kBigThreads, psmem, ctx->stream>>>(
-                in.v, in.p, mask, shift1, P1, d_idx, cur1, (uint64_t *)nullptr, ctx->d_ctr, 0);
-    })));
+    TRY(l1_scatter_seq(ctx, seq->layout, in.v, in.p, in.filtered, k, plan->bits1, d_idx, cur1, nullptr, 0));
     TRY(fetch_counters(ctx)); /* synchronises: every store of this rank has been issued and retired */
     if (rows_kept) *rows_kept = ctx->h_ctr[C_TOTAL];
     if (side_rows) *side_rows = ctx->h_ctr[C_SIDE];
@@ -2874,38 +2819,16 @@ extern "C" int dnagpu_shuffle_scatter_to(dnagpu_ctx *ctx, const dnagpu_seq *seq,
 }
 
 /* the same two steps from a key list on the device */
-static int shuffle_root(dnagpu_ctx *ctx, Scratch &sc, uint64_t n, uint64_t tile, uint64_t **root_off, uint64_t **tiles)
-{
-    TRY(sc.get((void **)root_off, 2 * 8));
-    ctx->h_ctr[0] = 0;
-    ctx->h_ctr[1] = n;
-    CU(ctx, cudaMemcpyAsync(*root_off, ctx->h_ctr, 16, cudaMemcpyHostToDevice, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream)); /* h_ctr is pinned staging shared with the counters */
-    return part_tiles(ctx, sc, *root_off, *root_off + 1, 1, tile, tiles);
-}
-
 extern "C" int dnagpu_shuffle_hist_keys(dnagpu_ctx *ctx, const uint64_t *d_keys, uint64_t n,
                                         const dnagpu_shuffle_plan *plan, uint64_t *digit_counts)
 {
     if (!ctx || !plan || !digit_counts || (n && !d_keys))
         return fail(ctx, DNAGPU_EARG, "dnagpu_shuffle_hist_keys: NULL argument");
     CU(ctx, cudaSetDevice(ctx->device));
-    for (uint32_t d = 0; d < plan->n_digits; ++d) digit_counts[d] = 0;
-    if (n == 0) return DNAGPU_OK;
-    Scratch sc(ctx);
-    const uint32_t P1 = plan->n_digits;
-    unsigned long long *hist1;
-    uint64_t *root_off, *tiles;
-    TRY(sc.get((void **)&hist1, (uint64_t)P1 * 8));
-    CU(ctx, cudaMemsetAsync(hist1, 0, (uint64_t)P1 * 8, ctx->stream));
-    TRY(shuffle_root(ctx, sc, n, kSuperTile, &root_off, &tiles));
-    TRY(launch(ctx, "part_hist", [&] {
-        k_part_hist_keys<<<grid_for(n, kSuperTile), kThreads, 0, ctx->stream>>>(d_keys, root_off, root_off + 1, tiles, 1, 1,
-                                                                              64 - plan->bits1, P1, hist1);
-    }));
-    CU(ctx, cudaMemcpyAsync(digit_counts, hist1, (uint64_t)P1 * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream));
-    return DNAGPU_OK;
+    CountInput in;
+    in.d_keys = d_keys;
+    in.n = n;
+    return shuffle_hist(ctx, in, 0, plan, digit_counts);
 }
 
 extern "C" int dnagpu_shuffle_scatter_keys_to(dnagpu_ctx *ctx, const uint64_t *d_keys, uint64_t n,
@@ -2918,25 +2841,12 @@ extern "C" int dnagpu_shuffle_scatter_keys_to(dnagpu_ctx *ctx, const uint64_t *d
     if (side_rows) *side_rows = 0;
     if (n == 0) return DNAGPU_OK;
     Scratch sc(ctx);
-    const uint32_t P1 = plan->n_digits;
-    std::vector<uint64_t> idx(P1); /* addresses / 8 as indices from a NULL base, as in dnagpu_shuffle_scatter_to */
-    for (uint32_t d = 0; d < P1; ++d) {
-        if (digit_dest[d] & 7) return fail(ctx, DNAGPU_EARG, "destination of digit %u is not 8-byte aligned", d);
-        idx[d] = digit_dest[d] >> 3;
-    }
-    uint64_t *d_idx, *root_off, *tiles;
+    uint64_t *d_idx, *root;
     unsigned long long *cur1;
-    TRY(sc.get((void **)&d_idx, ((uint64_t)P1 + 1) * 8));
-    TRY(sc.get((void **)&cur1, (uint64_t)P1 * 8));
-    CU(ctx, cudaMemcpyAsync(d_idx, idx.data(), (uint64_t)P1 * 8, cudaMemcpyHostToDevice, ctx->stream));
-    CU(ctx, cudaMemsetAsync(cur1, 0, (uint64_t)P1 * 8, ctx->stream));
-    TRY(shuffle_root(ctx, sc, n, 2 * kTileKeys, &root_off, &tiles)); /* synchronises: idx is a host temporary */
+    TRY(peer_dest(ctx, sc, plan, digit_dest, &d_idx, &cur1));
+    TRY(root_range(ctx, sc, n, &root));
     TRY(zero_counters(ctx));
-    const int psmem32 = 32 * kScatThreads * (int)sizeof(uint64_t) + (int)sizeof(ScatterSmem);
-    TRY(launch(ctx, "part_scatter_peer", [&] {
-        k_part_scatter_keys<true, kBigPerKeys, kBigThreadsKeys><<<grid_for(n, 2 * kTileKeys), kBigThreadsKeys, psmem32, ctx->stream>>>(
-            d_keys, root_off, root_off + 1, tiles, 1, 1, 64 - plan->bits1, P1, d_idx, cur1, (uint64_t *)nullptr, ctx->d_ctr);
-    }));
+    TRY(l1_scatter_keys(ctx, sc, d_keys, n, root, true, plan->bits1, d_idx, cur1, nullptr, 0));
     TRY(fetch_counters(ctx)); /* synchronises: every store of this rank has been issued and retired */
     if (side_rows) *side_rows = ctx->h_ctr[C_SIDE];
     return DNAGPU_OK;

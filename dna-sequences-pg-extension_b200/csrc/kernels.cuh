@@ -128,12 +128,9 @@ __device__ __forceinline__ bool pred_ok(const Pred &p, uint64_t x)
 
 __device__ __forceinline__ uint64_t ld_nc(const uint64_t *p) { return __ldg(p); }
 
-#ifndef DNAGPU_EXTRACT_ST
-#define DNAGPU_EXTRACT_ST "st.global.cs.v2.u64"
-#endif
 __device__ __forceinline__ void st_cs_v2(uint64_t *p, uint64_t a, uint64_t b)
 {
-    asm volatile(DNAGPU_EXTRACT_ST " [%0], {%1, %2};" ::"l"(p), "l"(a), "l"(b) : "memory");
+    asm volatile("st.global.cs.v2.u64 [%0], {%1, %2};" ::"l"(p), "l"(a), "l"(b) : "memory");
 }
 __device__ __forceinline__ void st_cs(uint64_t *p, uint64_t a)
 {
@@ -285,10 +282,7 @@ __device__ __forceinline__ uint32_t block_exscan(uint32_t v, uint32_t *total)
  * Each thread produces kPairs pairs of consecutive rows; a warp's store
  * instruction writes 512 contiguous bytes.  8 B written + 0.25 B read per row.
  * ================================================================================= */
-#ifndef DNAGPU_EXTRACT_PAIRS
-#define DNAGPU_EXTRACT_PAIRS 4
-#endif
-constexpr int kPairsPerThread = DNAGPU_EXTRACT_PAIRS;
+constexpr int kPairsPerThread = 4;
 
 template <int L>
 __global__ void __launch_bounds__(kThreads) k_extract(SeqView sv, uint64_t mask,
@@ -326,10 +320,7 @@ __global__ void __launch_bounds__(kThreads) k_extract(SeqView sv, uint64_t mask,
 
 /* The same with 256-bit stores (sm_100: STG.E.ENL2.256): one thread = FOUR consecutive rows = one full
  * 32-byte sector, a warp's store instruction writes 1 KB.  Needs a 32-byte aligned output. */
-#ifndef DNAGPU_EXTRACT_QUADS
-#define DNAGPU_EXTRACT_QUADS 2
-#endif
-constexpr int kQuadsPerThread = DNAGPU_EXTRACT_QUADS;
+constexpr int kQuadsPerThread = 2;
 
 __device__ __forceinline__ void st_v4(uint64_t *p, uint64_t a, uint64_t b, uint64_t c, uint64_t d)
 {
@@ -554,17 +545,11 @@ __device__ __forceinline__ uint32_t sa_word(uint64_t w, uint32_t lut_sa, uint32_
         const uint32_t addr = ((s >= 2 ? h >> (s - 2) : h << 2) & 12u) | lut_sa;
         uint32_t m;
         asm("ld.shared.u32 %0, [%1];" : "=r"(m) : "r"(addr));
-#ifdef DNAGPU_SA_ALU
-        const uint32_t t = F & m;
-        F = t + t + inj;
-        e = __funnelshift_l(t, e, 1); /* shifts the sign bit of t in at bit 0: step j ends at bit 31 - j */
-#else
         const uint32_t t = (F | inj) & m; /* F carries 2t of the step before; bit 32 - k of it is never set */
         uint64_t p;
         asm("mul.wide.u32 %0, %1, %2;" : "=l"(p) : "r"(t), "r"(two));
         F = (uint32_t)p;
         asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(e) : "r"(e), "r"(two), "r"((uint32_t)(p >> 32)));
-#endif
     }
     return __brev(e);
 }
@@ -603,11 +588,7 @@ __device__ __forceinline__ void sa_run_masks(const SeqView &sv, uint32_t lut, ui
     const int n_items = (int)((valid + 31) >> 5);
 #pragma unroll
     for (int i = 0; i <= kSaItems; ++i) w[i] = i <= n_items ? ld_nc(p + i) : 0; /* + the halo word */
-#ifdef DNAGPU_SA_ALU
-    uint32_t F = inj, e[kSaItems + 1];
-#else
     uint32_t F = 0, e[kSaItems + 1]; /* the injected bit is OR-ed in at the start of every step */
-#endif
 #pragma unroll
     for (int i = 0; i <= kSaItems; ++i) e[i] = i <= n_items ? sa_word(w[i], lut, inj, two, F) : 0u;
 #pragma unroll

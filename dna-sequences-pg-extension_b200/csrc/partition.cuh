@@ -10,7 +10,7 @@
  *
  *   level 1   k-mers (from packed words, WHERE fused) or a key list -> P1 <= 2048
  *             partitions by the top bits of mix64(kmer): histogram pass (exact sizes,
- *             no slack, no overflow), then scatter: a CTA ranks a tile of 8192 keys by
+ *             no slack, no overflow), then scatter: a CTA ranks a tile of 8192 or 16384 keys by
  *             partition in shared memory and writes one contiguous run per partition.
  *   level 2   the same inside every partition on the next hash bits (P2 <= 2048), so
  *             that a bucket holds ~1-3 K keys.  Skipped when level 1 is already enough.
@@ -41,12 +41,9 @@ constexpr int kMaxFan = 2048;              /* partitions per level              
  * which measured 2.5 % faster there than 1024 x 16 (17.46 vs 17.90 ms). */
 constexpr int kBigPer = 16, kBigThreads = 1024;        /* k_part_scatter_seq  */
 constexpr int kBigPerKeys = 32, kBigThreadsKeys = 512; /* k_part_scatter_keys */
-#ifndef DNAGPU_BUCKET_SLOTS
-#define DNAGPU_BUCKET_SLOTS 4096
-#endif
-constexpr int kBucketSlots = DNAGPU_BUCKET_SLOTS; /* shared-memory table of the count kernel (power of two) */
-constexpr int kBucketSlotBits = kBucketSlots == 4096 ? 12 : kBucketSlots == 8192 ? 13 : kBucketSlots == 2048 ? 11 : -1;
-static_assert(kBucketSlotBits > 0, "DNAGPU_BUCKET_SLOTS must be 2048, 4096 or 8192");
+constexpr int kBucketSlots = 4096; /* shared-memory table of the count kernel (power of two) */
+constexpr int kBucketSlotBits = 12;
+static_assert((1 << kBucketSlotBits) == kBucketSlots, "kBucketSlotBits must be log2(kBucketSlots)");
 constexpr uint64_t kSlotMul = 0x9E3779B97F4A7C15ull;
 constexpr uint64_t kPartMul = 0xD6E8FEB86659FD93ull;
 
@@ -307,14 +304,13 @@ __device__ __forceinline__ void scatter_flush(const ScatterSmem &s, const uint64
     }
 }
 
-/* one thread = PER consecutive start positions of one packed word (PER = 16: half an item, a tile of
- * 8192 keys, two CTAs per SM; PER = 32: a whole item, a tile of 16384 keys, one CTA per SM -- twice the
- * run length per (tile, digit), used when the runs are stored into peer memory over NVLink).
+/* the 16384-key tile of kBigThreads threads: one thread = PER = kBigPer consecutive start positions, half
+ * a packed word; one CTA per SM.
  * Straight-line code: a key that is not scattered (past the end, rejected by the WHERE
  * clause, or the k = 32 sentinel) is ranked into the dummy bin cur[fan] and its stores
  * are predicated off, so the unrolled loops carry no branches. */
-template <int L, bool FILTER, int PER = kScatPer, int THREADS = kScatThreads>
-__global__ void __launch_bounds__(THREADS, (PER * THREADS == 8192 ? 2 : 1)) k_part_scatter_seq(SeqView sv, Pred p, uint64_t mask, int shift,
+template <int L, bool FILTER>
+__global__ void __launch_bounds__(kBigThreads, 1) k_part_scatter_seq(SeqView sv, Pred p, uint64_t mask, int shift,
                                                                       uint32_t fan,
                                                                       const uint64_t *__restrict__ child_off,
                                                                       unsigned long long *__restrict__ child_cur,
@@ -322,16 +318,10 @@ __global__ void __launch_bounds__(THREADS, (PER * THREADS == 8192 ? 2 : 1)) k_pa
                                                                       unsigned long long *__restrict__ ctr,
                                                                       uint64_t cap)
 {
+    constexpr int PER = kBigPer, THREADS = kBigThreads;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     uint64_t *stage = reinterpret_cast<uint64_t *>(smem_raw);
     ScatterSmem &s = *reinterpret_cast<ScatterSmem *>(smem_raw + sizeof(uint64_t) * (PER * THREADS));
-#ifdef DNAGPU_PHASE_TIMING
-    long long tq[6];
-    tq[0] = clock64();
-#define PHASE_MARK(i) tq[i] = clock64()
-#else
-#define PHASE_MARK(i)
-#endif
     for (uint32_t i = threadIdx.x; i <= fan; i += THREADS) s.cur[i] = 0;
     __syncthreads();
     const uint32_t fm = fan - 1;
@@ -370,12 +360,9 @@ __global__ void __launch_bounds__(THREADS, (PER * THREADS == 8192 ? 2 : 1)) k_pa
             nxt >>= 2;
         }
     }
-    PHASE_MARK(1);
     __syncthreads();
-    PHASE_MARK(2);
     ScatterClaimT<THREADS> cl;
     const uint32_t total = scatter_plan<THREADS>(s, fan, child_cur, cl);
-    PHASE_MARK(3);
     {
         uint64_t cur = a0, nxt = a1;
 #pragma unroll
@@ -391,15 +378,7 @@ __global__ void __launch_bounds__(THREADS, (PER * THREADS == 8192 ? 2 : 1)) k_pa
     }
     scatter_publish<THREADS>(s, fan, child_off, cl, cap, ctr);
     __syncthreads();
-    PHASE_MARK(4);
     scatter_flush<PER, THREADS>(s, stage, total, shift, fm, out);
-    PHASE_MARK(5);
-#ifdef DNAGPU_PHASE_TIMING
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < 5; ++i) atomicAdd(&ctr[100 + i], (unsigned long long)(tq[i + 1] - tq[i]));
-        atomicAdd(&ctr[105], 1ull);
-    }
-#endif
     kept = warp_sum32(kept);
     side = warp_sum32(side);
     if ((threadIdx.x & 31) == 0) {
@@ -853,14 +832,7 @@ __global__ void __launch_bounds__(kThreads) k_count_buckets(const uint64_t *__re
             pre[u] = i < end ? ld_nc(keys + i) : kEmpty;
         }
     }
-#ifdef DNAGPU_PHASE_TIMING
-    long long ph[4] = {0, 0, 0, 0}, nbk = 0;
-#define CT_MARK(v) long long v = clock64()
-#else
-#define CT_MARK(v)
-#endif
     while (b < n_buckets) {
-        CT_MARK(c0);
         const uint64_t nb = b + gridDim.x;
         uint64_t nbeg = 0, nend = 0;
         if (nb < n_buckets) {
@@ -878,9 +850,7 @@ __global__ void __launch_bounds__(kThreads) k_count_buckets(const uint64_t *__re
             for (int i = 0; i < kBucketSlots * (int)sizeof(CT) / 16 / kThreads; ++i)
                 c4[i * kThreads + threadIdx.x] = make_uint4(0, 0, 0, 0);
         }
-        CT_MARK(c1);
         __syncthreads();
-        CT_MARK(c2);
         /* EMIT re-runs the count: rows of spilled keys come from the spill table itself.
          * The shared-memory CAS pipe is what bounds this kernel, and a CAS issued for one lane costs as
          * much as one issued for 32.  So probing is organised in ROUNDS: first probes of all prefetched
@@ -944,7 +914,6 @@ __global__ void __launch_bounds__(kThreads) k_count_buckets(const uint64_t *__re
         }
         for (uint64_t i = beg + (uint64_t)kPre * kThreads + threadIdx.x; i < end; i += kThreads)
             bucket_insert(tk, tc, ld_nc(keys + i), !EMIT, spill, spill_cap, bt, ty, ctr);
-        CT_MARK(c3);
         /* next bucket's keys fly while this one drains and the table is re-initialised */
 #pragma unroll
         for (int u = 0; u < kPre; ++u) {
@@ -952,12 +921,6 @@ __global__ void __launch_bounds__(kThreads) k_count_buckets(const uint64_t *__re
             pre[u] = i < nend ? ld_nc(keys + i) : kEmpty;
         }
         __syncthreads();
-#ifdef DNAGPU_PHASE_TIMING
-        {
-            long long c4 = clock64();
-            ph[0] += c1 - c0; ph[1] += c2 - c1; ph[2] += c3 - c2; ph[3] += c4 - c3; nbk++;
-        }
-#endif
         if (EMIT) {
             uint32_t mine = 0;
             for (int i = threadIdx.x; i < kBucketSlots; i += kThreads) mine += (tk[i] != kEmpty);
@@ -978,12 +941,6 @@ __global__ void __launch_bounds__(kThreads) k_count_buckets(const uint64_t *__re
         beg = nbeg;
         end = nend;
     }
-#ifdef DNAGPU_PHASE_TIMING
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < 4; ++i) atomicAdd(&ctr[110 + i], (unsigned long long)ph[i]);
-        atomicAdd(&ctr[114], (unsigned long long)nbk);
-    }
-#endif
     uint32_t d = warp_sum32(bt.distinct);
     int32_t u = (int32_t)__reduce_add_sync(0xffffffffu, bt.unique);
     if ((threadIdx.x & 31) == 0) {

@@ -8,7 +8,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# DNAGPU_LIB names another build of the same library (the -DDNAGPU_TUNING build the profiling scripts use)
+# DNAGPU_LIB names another build of the same library, e.g. to compare two builds on the same inputs
 LIB_PATH = os.environ.get("DNAGPU_LIB") or os.path.join(os.path.dirname(_HERE), "libdnagpu.so")
 
 u64 = C.c_uint64

@@ -3,7 +3,7 @@
 #   tools/sass_excerpt.sh > profiles/r02_sass_hot_kernels.txt
 SO=dna-sequences-pg-extension_b200/libdnagpu.so
 echo "# cuobjdump -sass of $SO (sm_100a), $(date -u +%F); nvcc $(nvcc --version | grep release | sed 's/.*release //')"
-for pat in 'k_extract4ILi0' 'k_part_scatter_seqILi0ELb0ELi16' 'k_part_scatter_keysILb0ELi32' 'k_count_buckets_bins' \
+for pat in 'k_extract4ILi0' 'k_part_scatter_seqILi0ELb0E' 'k_part_scatter_keysILb0ELi32' 'k_count_buckets_bins' \
            'k_collect_ownedILi4ELi3ELb0' 'k_collect_ownedILi4ELi0ELb0' 'k_filter_saILi1' 'k_filter_collectILi1'; do
   fn=$(cuobjdump -sass $SO 2>/dev/null | grep "Function :" | grep "$pat" | head -1 | sed 's/.*Function : //')
   [ -z "$fn" ] && continue
