@@ -42,6 +42,11 @@ struct dnagpu_ctx {
     unsigned long long *d_ctr = nullptr; /* C_COUNT + kMaxParts*2 u64 device counters */
     int bins_ctas_per_sm = 4;            /* resident CTAs of k_count_buckets_bins (occupancy query) */
     unsigned long long *h_ctr = nullptr; /* pinned mirror */
+    /* the abundance spectrum of the running query (dnagpu_count_spectrum): kSpecCum + spec_h u64 (kernels.cuh), grown on
+     * demand; spec_h = 0 outside such a query.  spec_side = the copies of 'G' x 32 (k = 32), a group of its own. */
+    unsigned long long *d_spec = nullptr;
+    uint32_t spec_alloc = 0, spec_h = 0;
+    uint64_t spec_side = 0;
     cudaStream_t copy_stream = nullptr; /* H2D of the host-buffer calls, overlapped with level 1 */
     /* dnagpu_create_multi: the contexts of devices[1..] (this one is devices[0]) and one shard buffer per GPU */
     std::vector<dnagpu_ctx *> peers;
@@ -305,7 +310,7 @@ extern "C" int dnagpu_create(dnagpu_ctx **out, int device)
 #undef PSMEM_ATTR
         {
             int per_sm = 0;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_count_buckets_bins, kThreads, 0) == cudaSuccess &&
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_count_buckets_bins<false>, kThreads, 0) == cudaSuccess &&
                 per_sm > 0)
                 ctx->bins_ctas_per_sm = per_sm;
         }
@@ -316,6 +321,10 @@ extern "C" int dnagpu_create(dnagpu_ctx **out, int device)
         cudaFuncSetAttribute(k_count_buckets<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bsmem);
         cudaFuncSetAttribute(k_count_buckets<false, unsigned long long>, cudaFuncAttributeMaxDynamicSharedMemorySize, bsmem64);
         cudaFuncSetAttribute(k_count_buckets<true, unsigned long long>, cudaFuncAttributeMaxDynamicSharedMemorySize, bsmem64);
+        cudaFuncSetAttribute(k_count_buckets<false, uint32_t, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             bsmem + kSpecSmem);
+        cudaFuncSetAttribute(k_count_buckets<false, unsigned long long, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             bsmem64 + kSpecSmem);
     }
     CU(nullptr, cudaGetLastError());
     *out = ctx;
@@ -402,6 +411,7 @@ extern "C" void dnagpu_destroy(dnagpu_ctx *ctx)
         cudaEventDestroy(r.e1);
     }
     if (ctx->d_ctr) cudaFree(ctx->d_ctr);
+    if (ctx->d_spec) cudaFree(ctx->d_spec);
     if (ctx->h_ctr) cudaFreeHost(ctx->h_ctr);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -1249,10 +1259,16 @@ extern "C" int dnagpu_filter_keys(dnagpu_ctx *ctx, const uint64_t *d_keys, uint6
 }
 
 /* ---- GROUP BY kmer ---------------------------------------------------------------------- */
+/* the spectrum starts over with the counters: every count, and every redo of one, begins here */
+static int zero_spectrum(dnagpu_ctx *ctx)
+{
+    if (ctx->spec_h) CU(ctx, cudaMemsetAsync(ctx->d_spec, 0, (kSpecCum + (uint64_t)ctx->spec_h) * 8, ctx->stream));
+    return DNAGPU_OK;
+}
 static int zero_counters(dnagpu_ctx *ctx)
 {
     CU(ctx, cudaMemsetAsync(ctx->d_ctr, 0, (C_COUNT + 2 * kMaxParts) * 8, ctx->stream));
-    return DNAGPU_OK;
+    return zero_spectrum(ctx);
 }
 static int fetch_counters(dnagpu_ctx *ctx)
 {
@@ -1347,7 +1363,11 @@ static int count_dense_t(dnagpu_ctx *ctx, const CountInput &in, int k, dnagpu_st
     }
     const unsigned sgrid = (unsigned)std::min<uint64_t>(grid_for(bins, kThreads), (uint64_t)ctx->sm_count * 16);
     TRY(launch(ctx, "dense_stats", [&] {
-        k_dense_stats<CT><<<sgrid, kThreads, 0, ctx->stream>>>(tab, bins, ctx->d_ctr);
+        if (ctx->spec_h)
+            k_dense_stats<CT, true><<<sgrid, kThreads, kSpecSmem, ctx->stream>>>(tab, bins, ctx->d_ctr,
+                                                                                ctx->d_spec + kSpecCum, ctx->spec_h);
+        else
+            k_dense_stats<CT><<<sgrid, kThreads, 0, ctx->stream>>>(tab, bins, ctx->d_ctr);
     }));
     TRY(fetch_counters(ctx));
     if (ctx->h_ctr[C_OVERFLOW]) return fail(ctx, DNAGPU_EARG, "a key is not a %d-mer (>= 4^k)", k);
@@ -1369,6 +1389,16 @@ static int count_dense_any(dnagpu_ctx *ctx, const CountInput &in, int k, dnagpu_
 {
     return in.n < 0xffffffffull ? count_dense_t<uint32_t>(ctx, in, k, stats, table)
                                 : count_dense_t<unsigned long long>(ctx, in, k, stats, table);
+}
+
+/* a spectrum query bins the final counts of a hash table (the HBM table, the bucket count's spill table) */
+static int table_spectrum(dnagpu_ctx *ctx, const Slot *slots, uint64_t cap)
+{
+    if (!ctx->spec_h) return DNAGPU_OK;
+    const unsigned grid = (unsigned)std::min<uint64_t>(grid_for(cap, kThreads), (uint64_t)ctx->sm_count * 8);
+    return launch(ctx, "table_spectrum", [&] {
+        k_table_spectrum<<<grid, kThreads, kSpecSmem, ctx->stream>>>(slots, cap, ctx->d_spec + kSpecCum, ctx->spec_h);
+    });
 }
 
 static int count_hash(dnagpu_ctx *ctx, const CountInput &in, int k, const dnagpu_count_opts *opts,
@@ -1413,7 +1443,9 @@ static int count_hash(dnagpu_ctx *ctx, const CountInput &in, int k, const dnagpu
     if (ctx->h_ctr[C_OVERFLOW])
         return fail(ctx, DNAGPU_EINTERNAL, "hash table of %llu slots overflowed (expected_keys too small)",
                     (unsigned long long)cap);
+    TRY(table_spectrum(ctx, slots, cap));
     const uint64_t side = ctx->h_ctr[C_SIDE]; /* 'G' x 32, the one key equal to the sentinel */
+    ctx->spec_side = side;
     const uint64_t in_table = ctx->h_ctr[C_DISTINCT];
     stats->total = ctx->h_ctr[C_TOTAL];
     stats->distinct = in_table + (side > 0);
@@ -1633,13 +1665,14 @@ static int part_level1(dnagpu_ctx *ctx, Scratch &sc, const CountInput &in, int k
 
 /* k_count_buckets over n keys in all: one key can occur n times, so past 2^32 - 1 keys the per-slot extras
  * counter is 64-bit (like count_dense_any's counters); every smaller call runs the 32-bit kernel */
-template <bool EMIT, class... A>
+template <bool EMIT, bool SPEC = false, class... A>
 static void launch_count_buckets(dnagpu_ctx *ctx, uint64_t n, unsigned grid, A... a)
 {
+    const int spec_smem = SPEC ? kSpecSmem : 0;
     if (n < 0xffffffffull)
-        k_count_buckets<EMIT, uint32_t><<<grid, kThreads, kBucketSlots * 12, ctx->stream>>>(a...);
+        k_count_buckets<EMIT, uint32_t, SPEC><<<grid, kThreads, kBucketSlots * 12 + spec_smem, ctx->stream>>>(a...);
     else
-        k_count_buckets<EMIT, unsigned long long><<<grid, kThreads, kBucketSlots * 16, ctx->stream>>>(a...);
+        k_count_buckets<EMIT, unsigned long long, SPEC><<<grid, kThreads, kBucketSlots * 16 + spec_smem, ctx->stream>>>(a...);
 }
 
 /* Level 2 (inside every parent; parents with equal parent % n_groups merge into the same children)
@@ -1731,13 +1764,24 @@ static int part_finish_impl(dnagpu_ctx *ctx, Scratch &sc, const uint64_t *keys, 
     TRY(sc.get((void **)&passed, n_buckets * 4 + 16));
     const unsigned bgrid = (unsigned)std::min<uint64_t>(n_buckets, (uint64_t)ctx->sm_count * ctx->bins_ctas_per_sm);
     TRY(launch(ctx, "count_buckets", [&] {
-        k_count_buckets_bins<<<bgrid, kThreads, 0, ctx->stream>>>(bucket_keys, bucket_off, bucket_end, n_buckets,
-                                                                 ctx->d_ctr, passed, ctx->d_ctr + C_PASSED);
+        if (ctx->spec_h)
+            k_count_buckets_bins<true><<<bgrid, kThreads, 0, ctx->stream>>>(bucket_keys, bucket_off, bucket_end, n_buckets,
+                                                                            ctx->d_ctr, passed, ctx->d_ctr + C_PASSED,
+                                                                            ctx->d_spec);
+        else
+            k_count_buckets_bins<<<bgrid, kThreads, 0, ctx->stream>>>(bucket_keys, bucket_off, bucket_end, n_buckets,
+                                                                     ctx->d_ctr, passed, ctx->d_ctr + C_PASSED);
     }));
     TRY(launch(ctx, "count_buckets_passed", [&] {
-        launch_count_buckets<false>(ctx, n, cgrid, bucket_keys, bucket_off, bucket_end, n_buckets, spill, spill_cap,
-                                    ctx->d_ctr, (uint64_t *)nullptr, (uint64_t *)nullptr, (const uint32_t *)passed,
-                                    (const unsigned long long *)ctx->d_ctr + C_PASSED);
+        if (ctx->spec_h)
+            launch_count_buckets<false, true>(ctx, n, cgrid, bucket_keys, bucket_off, bucket_end, n_buckets, spill,
+                                              spill_cap, ctx->d_ctr, (uint64_t *)nullptr, (uint64_t *)nullptr,
+                                              (const uint32_t *)passed, (const unsigned long long *)ctx->d_ctr + C_PASSED,
+                                              ctx->d_spec + kSpecCum, ctx->spec_h);
+        else
+            launch_count_buckets<false>(ctx, n, cgrid, bucket_keys, bucket_off, bucket_end, n_buckets, spill, spill_cap,
+                                        ctx->d_ctr, (uint64_t *)nullptr, (uint64_t *)nullptr, (const uint32_t *)passed,
+                                        (const unsigned long long *)ctx->d_ctr + C_PASSED);
     }));
     TRY(fetch_counters(ctx));
     if (ctx->h_ctr[C_L2OVF]) { /* some keys were dropped: the caller redoes level 2 exactly */
@@ -1746,7 +1790,9 @@ static int part_finish_impl(dnagpu_ctx *ctx, Scratch &sc, const uint64_t *keys, 
     }
     if (ctx->h_ctr[C_OVERFLOW])
         return fail(ctx, DNAGPU_EINTERNAL, "spill table of %llu slots overflowed", (unsigned long long)spill_cap);
+    TRY(table_spectrum(ctx, spill, spill_cap));
     const uint64_t side = ctx->h_ctr[C_SIDE];
+    ctx->spec_side = side;
     const uint64_t keyed = ctx->h_ctr[C_DISTINCT];
     stats->total = total_rows ? total_rows : ctx->h_ctr[C_TOTAL];
     stats->distinct = keyed + (side > 0);
@@ -1790,6 +1836,7 @@ static int part_finish(dnagpu_ctx *ctx, Scratch &sc, const uint64_t *keys, uint6
     CU(ctx, cudaMemsetAsync(ctx->d_ctr + C_DISTINCT, 0, 2 * 8, ctx->stream));
     CU(ctx, cudaMemsetAsync(ctx->d_ctr + C_OVERFLOW, 0, 2 * 8, ctx->stream));
     CU(ctx, cudaMemsetAsync(ctx->d_ctr + C_L2OVF, 0, 2 * 8, ctx->stream));
+    TRY(zero_spectrum(ctx));
     if (table && *table) {
         dnagpu_table_free(*table);
         *table = nullptr;
@@ -2259,11 +2306,54 @@ extern "C" int dnagpu_count_keys(dnagpu_ctx *ctx, const uint64_t *d_keys, uint64
     return count_any(ctx, in, k, opts, stats, table);
 }
 
+/* The abundance spectrum: the query dnagpu_count runs, with spec_h set so that every count method bins its final
+ * counts on the way (see kernels.cuh for the device layout).  Here the parts are added up:
+ *   cumulative part (k_count_buckets_bins):  groups of count c = C[c] - C[c+1] for c < H, count >= H = C[H];
+ *   direct part (every other kernel):         already binned by min(count, H);
+ *   'G' x 32 (k = 32):                        one group of count spec_side. */
+extern "C" int dnagpu_count_spectrum(dnagpu_ctx *ctx, const dnagpu_seq *seq, int k, const dnagpu_where *filter,
+                                     const dnagpu_count_opts *opts, uint32_t max_count, uint64_t *hist,
+                                     dnagpu_stats *stats)
+{
+    if (!ctx || !seq || !hist) return fail(ctx, DNAGPU_EARG, "dnagpu_count_spectrum: NULL argument");
+    if (max_count < 1 || max_count > kSpecMaxCount)
+        return fail(ctx, DNAGPU_EARG, "max_count must be between 1 and %u", kSpecMaxCount);
+    TRY(check_k(ctx, k));
+    TRY(check_filter_literals(ctx, filter));
+    CU(ctx, cudaSetDevice(ctx->device));
+    if (ctx->spec_alloc < max_count) {
+        if (ctx->d_spec) CU(ctx, cudaFree(ctx->d_spec));
+        ctx->d_spec = nullptr;
+        ctx->spec_alloc = 0;
+        CU(ctx, cudaMalloc((void **)&ctx->d_spec, (kSpecCum + (uint64_t)max_count) * 8));
+        ctx->spec_alloc = max_count;
+    }
+    struct SpecScope { /* the spectrum is wanted by this query only */
+        dnagpu_ctx *c;
+        ~SpecScope() { c->spec_h = 0; }
+    } spec_scope{ctx};
+    ctx->spec_h = max_count;
+    ctx->spec_side = 0;
+    TRY(zero_spectrum(ctx)); /* a count that finds no rows launches nothing */
+    dnagpu_stats st;
+    TRY(dnagpu_count(ctx, seq, k, filter, opts, &st, nullptr));
+    uint64_t cum[kSpecCum];
+    CU(ctx, cudaMemcpyAsync(cum, ctx->d_spec, sizeof cum, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(hist, ctx->d_spec + kSpecCum, (uint64_t)max_count * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    for (uint32_t c = 1; c < (uint32_t)kSpecCum && c <= max_count; ++c)
+        hist[c - 1] += c < max_count ? cum[c] - (c + 1 < (uint32_t)kSpecCum ? cum[c + 1] : 0) : cum[c];
+    if (ctx->spec_side) hist[std::min<uint64_t>(ctx->spec_side, max_count) - 1] += 1;
+    if (stats) *stats = st;
+    return DNAGPU_OK;
+}
+
 /* The host-buffer GROUP BY on every GPU of a multi context: shard d of the packed words goes to GPU d (H2D on
  * all PCIe links at once), then every GPU walks ALL shards through peer memory -- its own first, the others in
- * ring order -- and counts the k-mers it owns.  One host thread per GPU drives its (synchronous) count. */
+ * ring order -- and counts the k-mers it owns.  One host thread per GPU drives its (synchronous) count.  With
+ * max_count > 0 every GPU takes the spectrum of its share instead of a table, and the spectra add into hist. */
 static int count_kmers_multi(dnagpu_ctx *ctx, const uint64_t *words, uint64_t n_bases, int k, dnagpu_stats *stats,
-                             dnagpu_table **table)
+                             dnagpu_table **table, uint32_t max_count = 0, uint64_t *hist = nullptr)
 {
     const int G = 1 + (int)ctx->peers.size();
     std::vector<dnagpu_ctx *> cx(1, ctx);
@@ -2302,6 +2392,7 @@ static int count_kmers_multi(dnagpu_ctx *ctx, const uint64_t *words, uint64_t n_
     std::vector<int> rc((size_t)G, DNAGPU_OK);
     std::vector<dnagpu_stats> st((size_t)G);
     std::vector<dnagpu_table *> tb((size_t)G, nullptr);
+    std::vector<std::vector<uint64_t>> hs((size_t)G, std::vector<uint64_t>(max_count));
     std::vector<std::thread> th;
     for (int d = 0; d < G; ++d)
         th.emplace_back([&, d] {
@@ -2318,7 +2409,8 @@ static int count_kmers_multi(dnagpu_ctx *ctx, const uint64_t *words, uint64_t n_
             rc[d] = dnagpu_seq_wrap_pieces(cx[d], ptr, fb, ns, (uint32_t)G, n_bases, &seq);
             if (rc[d] != DNAGPU_OK) return;
             dnagpu_count_opts o = {DNAGPU_COUNT_AUTO, 0, 0.0, 0, (uint32_t)G, (uint32_t)d};
-            rc[d] = dnagpu_count(cx[d], seq, k, nullptr, &o, &st[d], table ? &tb[d] : nullptr);
+            rc[d] = max_count ? dnagpu_count_spectrum(cx[d], seq, k, nullptr, &o, max_count, hs[d].data(), &st[d])
+                              : dnagpu_count(cx[d], seq, k, nullptr, &o, &st[d], table ? &tb[d] : nullptr);
             dnagpu_seq_free(seq);
         });
     for (auto &t : th) t.join();
@@ -2333,6 +2425,11 @@ static int count_kmers_multi(dnagpu_ctx *ctx, const uint64_t *words, uint64_t n_
         stats->total += st[d].total;
         stats->distinct += st[d].distinct;
         stats->unique += st[d].unique;
+    }
+    if (max_count) {
+        std::fill(hist, hist + max_count, 0);
+        for (int d = 0; d < G; ++d)
+            for (uint32_t c = 0; c < max_count; ++c) hist[c] += hs[d][c];
     }
     if (table) {
         dnagpu_table *t = new (std::nothrow) dnagpu_table();
@@ -2373,6 +2470,27 @@ extern "C" int dnagpu_count_kmers(dnagpu_ctx *ctx, const uint64_t *words, uint64
     dnagpu_seq *seq = nullptr;
     TRY(dnagpu_seq_upload(ctx, words, n_bases, &seq));
     int rc = dnagpu_count(ctx, seq, k, filter, nullptr, stats, table);
+    dnagpu_seq_free(seq);
+    return rc;
+}
+
+extern "C" int dnagpu_count_kmers_spectrum(dnagpu_ctx *ctx, const uint64_t *words, uint64_t n_bases, int k,
+                                           const dnagpu_where *filter, uint32_t max_count, uint64_t *hist,
+                                           dnagpu_stats *stats)
+{
+    if (!ctx || !hist) return fail(ctx, DNAGPU_EARG, "dnagpu_count_kmers_spectrum: NULL argument");
+    if (max_count < 1 || max_count > kSpecMaxCount)
+        return fail(ctx, DNAGPU_EARG, "max_count must be between 1 and %u", kSpecMaxCount);
+    TRY(check_k(ctx, k));
+    TRY(check_filter_literals(ctx, filter));
+    if (!ctx->peers.empty() && words && (!filter || (filter->prefix_len == 0 && !filter->qkmer)) &&
+        rows_of(n_bases, k) >= (1ull << 21)) { /* the same fan-out rule as dnagpu_count_kmers */
+        dnagpu_stats local;
+        return count_kmers_multi(ctx, words, n_bases, k, stats ? stats : &local, nullptr, max_count, hist);
+    }
+    dnagpu_seq *seq = nullptr;
+    TRY(dnagpu_seq_upload(ctx, words, n_bases, &seq));
+    int rc = dnagpu_count_spectrum(ctx, seq, k, filter, nullptr, max_count, hist, stats);
     dnagpu_seq_free(seq);
     return rc;
 }

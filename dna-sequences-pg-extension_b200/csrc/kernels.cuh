@@ -910,6 +910,60 @@ __global__ void __launch_bounds__(kThreads) k_table_compact(const Slot *__restri
     }
 }
 
+/* ---- abundance spectrum: how many groups have count c, c = 1 .. H-1, and how many H or more ------------------
+ * Device layout of the histogram (u64): [0, kSpecCum) the cumulative part C[j] (k_count_buckets_bins: groups of count
+ * >= j, j = 1 .. 15), then H direct bins, bin c-1 for count min(c, H) (every kernel that sees a final count). */
+constexpr int kSpecCum = 16;
+constexpr uint32_t kSpecMaxCount = 1u << 20;
+constexpr uint32_t kSpecSmemBins = 1024; /* per-CTA shared bins of the small counts; the rest go to global atomics */
+constexpr int kSpecSmem = kSpecSmemBins * (int)sizeof(uint32_t);
+
+struct SpecBins {
+    uint32_t *s;             /* shared: s[c] for 1 <= c < n_s */
+    uint32_t n_s;
+    unsigned long long *hist; /* the direct bins */
+    uint32_t h;
+    __device__ __forceinline__ SpecBins(uint32_t *smem, unsigned long long *direct, uint32_t max_count)
+        : s(smem), n_s(min(max_count + 1, kSpecSmemBins)), hist(direct), h(max_count)
+    {
+    }
+    __device__ __forceinline__ void zero() /* the caller syncs */
+    {
+        for (uint32_t i = threadIdx.x; i < n_s; i += blockDim.x) s[i] = 0;
+    }
+    __device__ __forceinline__ void add(uint64_t c)
+    {
+        const uint32_t b = (uint32_t)min(c, (uint64_t)h);
+        if (b < n_s)
+            atomicAdd(&s[b], 1u);
+        else
+            atomicAdd(&hist[b - 1], 1ull);
+    }
+    __device__ __forceinline__ void flush() /* after a barrier */
+    {
+        for (uint32_t i = 1 + threadIdx.x; i < n_s; i += blockDim.x)
+            if (s[i]) atomicAdd(&hist[i - 1], (unsigned long long)s[i]);
+    }
+};
+
+/* the spectrum of a hash table (the HBM table of DNAGPU_COUNT_HASH, the spill table of the bucket count): every
+ * occupied slot holds its group's final count */
+__global__ void __launch_bounds__(kThreads) k_table_spectrum(const Slot *__restrict__ slots, uint64_t cap,
+                                                             unsigned long long *__restrict__ hist, uint32_t max_count)
+{
+    extern __shared__ uint32_t spec_smem[];
+    SpecBins sb(spec_smem, hist, max_count);
+    sb.zero();
+    __syncthreads();
+    const uint64_t stride = (uint64_t)gridDim.x * kThreads;
+    for (uint64_t i = (uint64_t)blockIdx.x * kThreads + threadIdx.x; i < cap; i += stride) {
+        const ulonglong2 v = __ldg(reinterpret_cast<const ulonglong2 *>(slots + i));
+        if (v.x != kEmpty) sb.add(v.y);
+    }
+    __syncthreads();
+    sb.flush();
+}
+
 /* =================================================================================
  * K3  GROUP BY kmer, dense variant: 4^k direct-indexed counters (k <= 16).
  *   k <= 7   per-CTA shared-memory histograms, replicated R ways by lane so that
@@ -1011,12 +1065,21 @@ __global__ void __launch_bounds__(kThreads) k_count_dense_keys(const uint64_t *_
     if ((threadIdx.x & 31) == 0 && total) atomicAdd(&ctr[C_TOTAL], (unsigned long long)total);
 }
 
-/* K5 for the dense table: distinct / unique, and optional compaction */
-template <typename CT>
+/* K5 for the dense table: distinct / unique, and optional compaction.  The SPEC form also bins every non-zero
+ * counter into the direct part of the spectrum (kSpecSmem bytes of dynamic shared memory). */
+template <typename CT, bool SPEC = false>
 __global__ void __launch_bounds__(kThreads) k_dense_stats(const CT *__restrict__ table,
                                                           uint64_t n_bins,
-                                                          unsigned long long *__restrict__ ctr)
+                                                          unsigned long long *__restrict__ ctr,
+                                                          unsigned long long *__restrict__ spec_direct = nullptr,
+                                                          uint32_t max_count = 0)
 {
+    extern __shared__ uint32_t spec_smem[];
+    SpecBins sb(spec_smem, spec_direct, max_count);
+    if constexpr (SPEC) {
+        sb.zero();
+        __syncthreads();
+    }
     uint64_t i = (uint64_t)blockIdx.x * kThreads + threadIdx.x;
     const uint64_t stride = (uint64_t)gridDim.x * kThreads;
     uint32_t d = 0, u = 0;
@@ -1024,6 +1087,12 @@ __global__ void __launch_bounds__(kThreads) k_dense_stats(const CT *__restrict__
         CT c = table[i];
         d += (c != 0);
         u += (c == 1);
+        if constexpr (SPEC)
+            if (c) sb.add((uint64_t)c);
+    }
+    if constexpr (SPEC) {
+        __syncthreads();
+        sb.flush();
     }
     d = warp_sum32(d);
     u = warp_sum32(u);

@@ -798,8 +798,11 @@ __device__ __forceinline__ void bucket_insert(unsigned long long *tk, CT *tc, ui
 }
 
 /* CT, the per-slot count of extra occurrences: uint32_t unless the call has 2^32 - 1 or more keys, where one key
- * can occur 2^32 + 1 times and a 32-bit count would wrap (unsigned long long, 16 bytes per slot) */
-template <bool EMIT, class CT = uint32_t>
+ * can occur 2^32 + 1 times and a 32-bit count would wrap (unsigned long long, 16 bytes per slot).
+ * SPEC (not with EMIT): a bucket's keys are all in that bucket, so once it has drained every occupied slot holds its
+ * group's final count; those are binned into the direct part of the spectrum (kSpecSmem more bytes of dynamic shared
+ * memory, after the table).  Spilled keys are binned from the spill table afterwards. */
+template <bool EMIT, class CT = uint32_t, bool SPEC = false>
 __global__ void __launch_bounds__(kThreads) k_count_buckets(const uint64_t *__restrict__ keys,
                                                             const uint64_t *__restrict__ bucket_off,
                                                             const uint64_t *__restrict__ bucket_end,
@@ -809,14 +812,20 @@ __global__ void __launch_bounds__(kThreads) k_count_buckets(const uint64_t *__re
                                                             uint64_t *__restrict__ out_kmers,
                                                             uint64_t *__restrict__ out_counts,
                                                             const uint32_t *__restrict__ list = nullptr,
-                                                            const unsigned long long *__restrict__ list_n = nullptr)
+                                                            const unsigned long long *__restrict__ list_n = nullptr,
+                                                            unsigned long long *__restrict__ spec_direct = nullptr,
+                                                            uint32_t max_count = 0)
 {
+    static_assert(!(EMIT && SPEC), "the emitting pass re-runs a count whose spectrum is already taken");
     /* with a list: only the buckets list[0 .. *list_n) (the ones k_count_buckets_bins passed on) */
     if (list) n_buckets = *list_n;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     unsigned long long *tk = reinterpret_cast<unsigned long long *>(smem_raw);                /* keys   */
     CT *tc = reinterpret_cast<CT *>(smem_raw + sizeof(uint64_t) * kBucketSlots); /* extras */
     __shared__ unsigned long long row_base;
+#define SPEC_BINS SpecBins(reinterpret_cast<uint32_t *>(smem_raw + (sizeof(uint64_t) + sizeof(CT)) * kBucketSlots), \
+                           spec_direct, max_count)
+    if constexpr (SPEC) SPEC_BINS.zero(); /* before the first barrier of the loop; flushed after the last */
     Tally ty = {0, 0, 0, 0}; /* spilled keys account themselves through hash_insert */
     BucketTally bt = {0, 0};
     uint64_t b = blockIdx.x;
@@ -937,10 +946,21 @@ __global__ void __launch_bounds__(kThreads) k_count_buckets(const uint64_t *__re
                 }
             __syncthreads();
         }
+        if constexpr (SPEC) {
+            SpecBins sb = SPEC_BINS;
+            for (int i = threadIdx.x; i < kBucketSlots; i += kThreads)
+                if (tk[i] != kEmpty) sb.add((uint64_t)tc[i] + 1);
+            __syncthreads(); /* before the next bucket clears the table */
+        }
         b = nb;
         beg = nbeg;
         end = nend;
     }
+    if constexpr (SPEC) {
+        __syncthreads();
+        SPEC_BINS.flush();
+    }
+#undef SPEC_BINS
     uint32_t d = warp_sum32(bt.distinct);
     int32_t u = (int32_t)__reduce_add_sync(0xffffffffu, bt.unique);
     if ((threadIdx.x & 31) == 0) {
@@ -1022,14 +1042,26 @@ __device__ __forceinline__ void bins_place(const uint64_t (&x)[kBinPer], const u
         else { constexpr int ROWS = kBinPer; CALL; }               \
     } while (0)
 
+/* SPEC also takes the cumulative spectrum C[j] (groups of count >= j) of the buckets it counts, into spec_cum[j]:
+ * a group of count m has exactly one key with e = j - 1 for each j = 1 .. m, so C[1] = keys - repeats, C[2] = second,
+ * and C[j >= 3] = keys with e = j - 1 (rare: repeated k-mers only).  A bin holds at most kBinHeavy keys: j <= 15. */
+template <bool SPEC = false>
 __global__ void __launch_bounds__(kThreads, 4) k_count_buckets_bins(const uint64_t *__restrict__ keys,
                                                                     const uint64_t *__restrict__ bucket_off,
                                                                     const uint64_t *__restrict__ bucket_end,
                                                                     uint64_t n_buckets,
                                                                     unsigned long long *__restrict__ ctr,
                                                                     uint32_t *__restrict__ list,
-                                                                    unsigned long long *__restrict__ list_n)
+                                                                    unsigned long long *__restrict__ list_n,
+                                                                    unsigned long long *__restrict__ spec_cum = nullptr)
 {
+    static_assert(kBinHeavy < kSpecCum, "the cumulative spectrum of a bin");
+    uint32_t *scum = nullptr; /* keys with e = j - 1 >= 2, by j */
+    if constexpr (SPEC) {
+        __shared__ uint32_t scum_s[kSpecCum];
+        scum = scum_s;
+        if (threadIdx.x < kSpecCum) scum[threadIdx.x] = 0; /* before the first barrier */
+    }
     /* every array ends in dummy entries, one per lane (+ 15 for a dummy's meaningless 4-bit rank): the lanes
      * past the end of a bucket's last row work on those instead of branching around the atomics and the stores */
     __shared__ __align__(16) uint64_t stage_raw[4 + kBinCap + 48]; /* 4 in front: the compare phase looks back */
@@ -1117,6 +1149,8 @@ __global__ void __launch_bounds__(kThreads, 4) k_count_buckets_bins(const uint64
                     }
                     repeats += e >= 1;
                     second += e == 1;
+                    if constexpr (SPEC)
+                        if (e >= 2) atomicAdd(&scum[e + 1], 1u);
                 }
             }
         }
@@ -1134,6 +1168,15 @@ __global__ void __launch_bounds__(kThreads, 4) k_count_buckets_bins(const uint64
     if (tid == 0 && placed) {
         atomicAdd(&ctr[C_DISTINCT], placed);
         atomicAdd(&ctr[C_UNIQUE], placed);
+    }
+    if constexpr (SPEC) {
+        if (lane == 0 && (repeats | second)) {
+            atomicAdd(&spec_cum[1], (unsigned long long)(-(long long)repeats));
+            atomicAdd(&spec_cum[2], (unsigned long long)second);
+        }
+        if (tid == 0 && placed) atomicAdd(&spec_cum[1], placed);
+        __syncthreads();
+        if (tid >= 3 && tid < kSpecCum && scum[tid]) atomicAdd(&spec_cum[tid], (unsigned long long)scum[tid]);
     }
 }
 

@@ -23,7 +23,7 @@ COUNT_FLAG_EXACT = 1  # DNAGPU_COUNT_FLAG_EXACT: exact two-pass partition levels
 MAX_K = 32
 
 __all__ = ["Context", "Seq", "Table", "Dna", "Kmer", "Qkmer", "DnaError", "KmerArray",
-           "generate_kmers", "filter_kmers", "count_kmers", "kmer_stats", "owner_of",
+           "generate_kmers", "filter_kmers", "count_kmers", "kmer_stats", "kmer_spectrum", "owner_of",
            "default_context", "QKMER_ALPHABET"]
 
 
@@ -554,6 +554,29 @@ class Context:
                                        C.byref(th) if table else None))
         return st, (Table(self, th) if table else None)
 
+    def count_spectrum(self, seq, k, prefix=None, pattern=None, max_count=10000, method=COUNT_AUTO, exact=False,
+                       owner=None, planes=False):
+        """The abundance spectrum of `count`'s query -> (Stats, uint64 array h of max_count entries): h[c-1] distinct
+        k-mers occur exactly c times (c < max_count), h[max_count-1] occur max_count times or more."""
+        w, _keep = _where(prefix, pattern, planes)
+        o = self._opts(method, 0.0, 0, exact, owner)
+        st, hist = Stats(), np.zeros(max(int(max_count), 1), dtype=np.uint64)
+        self._ok(self.lib.dnagpu_count_spectrum(self.handle, seq.handle, k, C.byref(w) if w is not None else None,
+                                                C.byref(o) if o is not None else None, max_count,
+                                                hist.ctypes.data, C.byref(st)))
+        return st, hist
+
+    def count_kmers_spectrum(self, dna, k, prefix=None, pattern=None, max_count=10000):
+        """Host in: `SELECT least(count, max_count), count(*) FROM (... GROUP BY kmer) GROUP BY 1` as count_spectrum
+        returns it.  On a multi-GPU context every GPU counts its share."""
+        dna = dna if isinstance(dna, Dna) else Dna(dna)
+        w, _keep = _where(prefix, pattern)
+        st, hist = Stats(), np.zeros(max(int(max_count), 1), dtype=np.uint64)
+        self._ok(self.lib.dnagpu_count_kmers_spectrum(self.handle, dna.words.ctypes.data, dna.length, k,
+                                                      C.byref(w) if w is not None else None, max_count,
+                                                      hist.ctypes.data, C.byref(st)))
+        return st, hist
+
     def count_keys(self, keys, k, table=False, method=COUNT_AUTO, load_factor=0.0, expected_keys=0):
         self._after_torch()
         o = self._opts(method, load_factor, expected_keys)
@@ -759,3 +782,11 @@ def kmer_stats(dna, k, prefix=None, pattern=None, ctx=None):
     """total / distinct / unique of README.md:122-130 -> (total, distinct, unique)."""
     st, _ = (ctx or default_context()).count_kmers(dna, k, prefix=prefix, pattern=pattern, table=False)
     return int(st.total), int(st.distinct), int(st.unique)
+
+
+def kmer_spectrum(dna, k, prefix=None, pattern=None, max_count=10000, ctx=None):
+    """The k-mer abundance spectrum -> uint64 array h: h[c-1] distinct k-mers occur c times, the last entry
+    max_count times or more (`SELECT least(count, max_count), count(*) ... GROUP BY 1`)."""
+    _, hist = (ctx or default_context()).count_kmers_spectrum(dna, k, prefix=prefix, pattern=pattern,
+                                                             max_count=max_count)
+    return hist

@@ -81,6 +81,10 @@ SIGNATURES = {
                                C.POINTER(Stats), C.POINTER(vp)]),
     "dnagpu_count_keys": (C.c_int, [vp, vp, u64, C.c_int, C.POINTER(CountOpts), C.POINTER(Stats),
                                     C.POINTER(vp)]),
+    "dnagpu_count_spectrum": (C.c_int, [vp, vp, C.c_int, C.POINTER(Where), C.POINTER(CountOpts), C.c_uint32,
+                                        vp, C.POINTER(Stats)]),
+    "dnagpu_count_kmers_spectrum": (C.c_int, [vp, vp, u64, C.c_int, C.POINTER(Where), C.c_uint32, vp,
+                                              C.POINTER(Stats)]),
     "dnagpu_table_rows": (u64, [vp]),
     "dnagpu_table_k": (C.c_int, [vp]),
     "dnagpu_table_fetch": (C.c_int, [vp, vp, u64, u64, vp, vp]),

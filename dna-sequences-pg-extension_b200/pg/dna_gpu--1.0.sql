@@ -28,6 +28,19 @@ CREATE OR REPLACE FUNCTION count_kmers(dna, integer, kmer, qkmer, OUT kmer kmer,
     AS 'MODULE_PATHNAME', 'count_kmers'
     LANGUAGE C IMMUTABLE PARALLEL SAFE;
 
+-- The k-mer abundance spectrum in one call: one row per non-zero bin, count = H meaning "H or more", i.e.
+--   SELECT least(count, H) AS count, count(*) AS kmers
+--   FROM (SELECT kmer, count(*) FROM generate_kmers(seq, k) AS k(kmer) [WHERE ...] GROUP BY kmer) g
+--   GROUP BY 1 ORDER BY 1;
+CREATE OR REPLACE FUNCTION kmer_spectrum(dna, integer, integer, OUT count bigint, OUT kmers bigint)
+    RETURNS SETOF record
+    AS 'MODULE_PATHNAME', 'kmer_spectrum'
+    LANGUAGE C IMMUTABLE STRICT PARALLEL SAFE;
+CREATE OR REPLACE FUNCTION kmer_spectrum(dna, integer, kmer, qkmer, integer, OUT count bigint, OUT kmers bigint)
+    RETURNS SETOF record
+    AS 'MODULE_PATHNAME', 'kmer_spectrum'
+    LANGUAGE C IMMUTABLE PARALLEL SAFE;
+
 -- The table form (test.sql:140-150) as an aggregate: one GPU query for the whole table.
 --   SELECT (kmer_stats_agg(sequence, 10)).* FROM dna_sequences;
 CREATE OR REPLACE FUNCTION kmer_stats_agg_trans(internal, dna, integer)

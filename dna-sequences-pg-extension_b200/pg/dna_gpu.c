@@ -14,6 +14,8 @@
  *       unique query (README.md:122-130) without ever materialising the k-mers in the executor.
  *   count_kmers(dna, int [, kmer, qkmer]) SETOF (kmer, count)   the GROUP BY of README.md:107-116; the grouped
  *       rows stay on the GPU and are fetched in windows.
+ *   kmer_spectrum(dna, int [, kmer, qkmer], int H) SETOF (count, kmers)   the abundance spectrum of that GROUP BY
+ *       (how many k-mers occur c times, the last row H or more times), binned on the GPU: H integers come back.
  *   kmer_stats_agg(dna, int)   aggregate: the table form of the query (test.sql:140-150,
  *       FROM dna_sequences d, generate_kmers(d.sequence, k) ... GROUP BY) in one pass over the table: the
  *       transition function appends every value to a ragged batch, the final function counts the batch on
@@ -416,6 +418,92 @@ count_kmers(PG_FUNCTION_ARGS)
         SRF_RETURN_NEXT(funcctx, HeapTupleGetDatum(heap_form_tuple((TupleDesc) funcctx->tuple_desc, values, nulls)));
     }
     count_state_release(st);
+    SRF_RETURN_DONE(funcctx);
+}
+
+/* =====================================================================================================
+ * kmer_spectrum(dna, int [, kmer, qkmer], int H) SETOF (count, kmers): the k-mer abundance spectrum,
+ *   SELECT least(count, H) AS count, count(*) AS kmers
+ *   FROM (SELECT kmer, count(*) FROM generate_kmers(seq, k) AS k(kmer) [WHERE ...] GROUP BY kmer) g
+ *   GROUP BY 1 ORDER BY 1;
+ * One row per non-zero bin in ascending count; count = H means "H or more".  The first call runs the whole query
+ * and keeps at most H rows in backend memory, so no GPU handle outlives it.
+ * ===================================================================================================== */
+typedef struct SpectrumState
+{
+    uint64_t   *count;
+    uint64_t   *kmers;
+    uint64_t    n, pos;
+} SpectrumState;
+
+PG_FUNCTION_INFO_V1(kmer_spectrum);
+Datum
+kmer_spectrum(PG_FUNCTION_ARGS)
+{
+    FuncCallContext *funcctx;
+    SpectrumState *st;
+    const int   h_arg = PG_NARGS() - 1;
+
+    if (PG_ARGISNULL(0) || PG_ARGISNULL(1) || PG_ARGISNULL(h_arg))
+    {
+        funcctx = SRF_IS_FIRSTCALL() ? SRF_FIRSTCALL_INIT() : SRF_PERCALL_SETUP();
+        SRF_RETURN_DONE(funcctx);
+    }
+    if (SRF_IS_FIRSTCALL())
+    {
+        MemoryContext oldcontext;
+        Dna        *dna;
+        int         k, rc;
+        int32       h;
+        uint64_t   *hist;
+        uint64_t    c;
+        dnagpu_stats stats;
+        dnagpu_where w;
+        const dnagpu_where *wp;
+        TupleDesc   tupdesc;
+
+        funcctx = SRF_FIRSTCALL_INIT();
+        oldcontext = MemoryContextSwitchTo(funcctx->multi_call_memory_ctx);
+        dna = (Dna *) PG_GETARG_VARLENA_P(0);
+        k = PG_GETARG_INT32(1);
+        h = PG_GETARG_INT32(h_arg);
+        check_k(k);
+        if (get_call_result_type(fcinfo, NULL, &tupdesc) != TYPEFUNC_COMPOSITE)
+            ereport(ERROR, (errmsg("kmer_spectrum must be called in a context that accepts a record")));
+        funcctx->tuple_desc = BlessTupleDesc(tupdesc);
+        wp = where_args(fcinfo, &w);
+        /* an H out of range is reported by the library; it writes nothing then */
+        hist = (uint64_t *) palloc0(sizeof(uint64_t) * (h >= 1 && h <= (1 << 20) ? (uint64_t) h : 1));
+        rc = dnagpu_count_kmers_spectrum(gpu(), dna->bit_sequence, dna->length, k, wp, (uint32_t) h, hist, &stats);
+        if (rc != DNAGPU_OK)
+            ereport(ERROR, (errmsg("%s", dnagpu_last_error(backend_ctx))));
+        st = (SpectrumState *) palloc0(sizeof(SpectrumState));
+        st->count = (uint64_t *) palloc(sizeof(uint64_t) * (uint64_t) h);
+        st->kmers = (uint64_t *) palloc(sizeof(uint64_t) * (uint64_t) h);
+        for (c = 1; c <= (uint64_t) h; c++)
+            if (hist[c - 1])
+            {
+                st->count[st->n] = c;
+                st->kmers[st->n] = hist[c - 1];
+                st->n++;
+            }
+        pfree(hist);
+        funcctx->user_fctx = st;
+        MemoryContextSwitchTo(oldcontext);
+    }
+
+    funcctx = SRF_PERCALL_SETUP();
+    st = (SpectrumState *) funcctx->user_fctx;
+    if (st->pos < st->n)
+    {
+        Datum       values[2];
+        bool        nulls[2] = {false, false};
+
+        values[0] = Int64GetDatum((int64) st->count[st->pos]);
+        values[1] = Int64GetDatum((int64) st->kmers[st->pos]);
+        st->pos++;
+        SRF_RETURN_NEXT(funcctx, HeapTupleGetDatum(heap_form_tuple((TupleDesc) funcctx->tuple_desc, values, nulls)));
+    }
     SRF_RETURN_DONE(funcctx);
 }
 

@@ -25,6 +25,9 @@
  *       (README.md:107-135, test.sql:95-119,140-154), i.e. PostgreSQL's
  *       HashAggregate driven by kmer_hash (dna.c:722-735) and kmer_eq
  *       (dna.c:655-668,686-696; opclass dna--1.0.sql:204-212).
+ *   dnagpu_count_kmers_spectrum / dnagpu_count_spectrum
+ *       SELECT least(count, H), count(*) FROM (... GROUP BY kmer) g GROUP BY 1: the abundance spectrum of
+ *       the same GROUP BY, binned on the GPU (unique is its first bin, distinct its sum).
  *   dnagpu_collect
  *       the same WHERE clauses when the row order does not matter (the input of
  *       a GROUP BY or of the exchange between GPUs): one predicate scan.
@@ -293,6 +296,21 @@ int dnagpu_count(dnagpu_ctx *ctx, const dnagpu_seq *seq, int k,
 int dnagpu_count_keys(dnagpu_ctx *ctx, const uint64_t *d_keys, uint64_t n, int k,
                       const dnagpu_count_opts *opts, dnagpu_stats *stats,
                       dnagpu_table **table);
+
+/* The abundance spectrum of the same query (jellyfish histo): with H = max_count, 1 <= H <= 2^20,
+ *   hist[c-1] = the number of distinct k-mers that occur exactly c times, c = 1 .. H-1;
+ *   hist[H-1] = the number that occur H times or more  (SQL: GROUP BY least(count, H)).
+ * hist is H uint64 in host memory.  stats receives what dnagpu_count returns, so sum(hist) == distinct and, for
+ * H >= 2, hist[0] == unique.  WHERE clause, layouts, methods, flags and the owner restriction are those of
+ * dnagpu_count; no table is built: the spectrum is binned on the device by the count itself, and H integers come
+ * back.  'G' x 32 (k = 32) is one group like any other.  A bad max_count or a NULL hist: DNAGPU_EARG. */
+int dnagpu_count_spectrum(dnagpu_ctx *ctx, const dnagpu_seq *seq, int k, const dnagpu_where *filter,
+                          const dnagpu_count_opts *opts, uint32_t max_count, uint64_t *hist, dnagpu_stats *stats);
+/* The same from host words (what the SQL glue calls).  On a dnagpu_create_multi context and without a WHERE clause,
+ * every GPU counts the k-mers it owns (as dnagpu_count_kmers does) and the spectra add. */
+int dnagpu_count_kmers_spectrum(dnagpu_ctx *ctx, const uint64_t *words, uint64_t n_bases, int k,
+                                const dnagpu_where *filter, uint32_t max_count, uint64_t *hist,
+                                dnagpu_stats *stats);
 
 /* The grouped result.  Rows are (kmer bits, count); order is unspecified (as
  * for a HashAggregate) but fixed for the life of the table. */
