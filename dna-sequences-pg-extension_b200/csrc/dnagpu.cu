@@ -1318,7 +1318,6 @@ static int pick_method(const dnagpu_count_opts *opts, int k, uint64_t n)
      * drop to 15-30 Gkmer/s, where partition + shared-memory count wins by > 5x. */
     if (k <= 12 && pow4_capped(k) <= std::max<uint64_t>(1ull << 16, 8 * n)) return DNAGPU_COUNT_DENSE;
     if (n >= (1ull << 21)) return DNAGPU_COUNT_PARTITION;
-    if (k <= 16 && pow4_capped(k) <= std::max<uint64_t>(1ull << 16, 8 * n)) return DNAGPU_COUNT_DENSE;
     return DNAGPU_COUNT_HASH;
 }
 
