@@ -2163,7 +2163,7 @@ static int count_owned(dnagpu_ctx *ctx, const dnagpu_seq *seq, int k, const dnag
         } else {
             const unsigned grid = (unsigned)std::min<uint64_t>(grid_for(n_vitems, kScatThreads), (uint64_t)ctx->sm_count * 8);
 #define OWNED_ANY(LIN) k_collect_owned_any<LIN><<<grid, kScatThreads, 0, ctx->stream>>>(ov, mask, own, cap, ctx->d_ctr + C_CURSOR, keys)
-            TRY(launch(ctx, "collect_owned", [&] {
+            TRY(launch(ctx, "collect_owned_any", [&] {
                 if (lin == 3) OWNED_ANY(3); else if (lin == 2) OWNED_ANY(2); else if (lin == 1) OWNED_ANY(1); else OWNED_ANY(0);
             }));
 #undef OWNED_ANY
@@ -2277,7 +2277,8 @@ extern "C" int dnagpu_count(dnagpu_ctx *ctx, const dnagpu_seq *seq, int k,
     TRY(check_k(ctx, k));
     TRY(check_filter_literals(ctx, filter));
     CU(ctx, cudaSetDevice(ctx->device));
-    if (opts && opts->owner_parts > 1) {
+    /* one owner of a sequence in pieces is the whole count of one GPU's ring; of a single sequence, no restriction */
+    if (opts && (opts->owner_parts > 1 || (opts->owner_parts == 1 && seq->layout == kPieces))) {
         if (filter && (filter->prefix_len || filter->qkmer))
             return fail(ctx, DNAGPU_EARG, "an owner restriction cannot be combined with a WHERE clause");
         if (opts->method != DNAGPU_COUNT_AUTO && opts->method != DNAGPU_COUNT_PARTITION)

@@ -488,18 +488,19 @@ struct OwnedView {
     uint32_t n_pieces;
 };
 
-/* What a kernel needs to tell its owner's k-mers: the hash range of the multiplicative form (lo, span), or for the
- * linear form the XOR seeds of the rank bits (inv[i] = ~0 when bit i of the rank is 0: the chain then ends in "bit
- * matches") and the taps in force (en, bit p: tap p lies inside the k-mer, i.e. own_tau(p) < 2k). */
+/* What a kernel needs to tell its owner's k-mers: the hash range of the multiplicative form (lo, span_m1 = its
+ * length - 1, so that one owner's whole range of 2^32 hashes fits), or for the linear form the XOR seeds of the
+ * rank bits (inv[i] = ~0 when bit i of the rank is 0: the chain then ends in "bit matches") and the taps in force
+ * (en, bit p: tap p lies inside the k-mer, i.e. own_tau(p) < 2k). */
 struct OwnRange {
-    uint32_t lo, span, en, inv[3];
+    uint32_t lo, span_m1, en, inv[3];
 };
 __host__ inline OwnRange own_range_of(uint32_t n_parts, uint32_t part, int k)
 {
     OwnRange r;
     const uint64_t lo = (((uint64_t)part << 32) + n_parts - 1) / n_parts, hi = (((uint64_t)(part + 1) << 32) + n_parts - 1) / n_parts;
     r.lo = (uint32_t)lo; /* owner r holds the hashes [ceil(r 2^32 / G), ceil((r + 1) 2^32 / G)): what (hash * G) >> 32 == r says */
-    r.span = (uint32_t)(hi - lo);
+    r.span_m1 = (uint32_t)(hi - lo - 1);
     r.en = 0;
     for (int p = 0; p < kOwnPool; ++p)
         if (own_tau(p) < 2 * k) r.en |= 1u << p;
@@ -523,7 +524,7 @@ __device__ __forceinline__ uint32_t owned_mask(uint64_t w0, uint32_t a2, uint32_
             const uint32_t lo = j == 0 ? a0 : j < 16 ? __funnelshift_r(a0, a1, 2 * j) : j == 16 ? a1
                                                                                                  : __funnelshift_r(a1, a2, 2 * j - 32);
             const uint32_t t = (MASKLO ? lo & mask_lo : lo) * kOwnerMul - own.lo;
-            km |= (uint32_t)(t < own.span) << j;
+            km |= (uint32_t)(t <= own.span_m1) << j;
         }
         return km;
     }

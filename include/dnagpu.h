@@ -142,7 +142,8 @@ typedef struct dnagpu_count_opts {
      * (0 parts = no restriction).  Every GPU of a box runs the same query over the same sequence --
      * resident as one piece per GPU, see dnagpu_seq_wrap_pieces -- with its own owner_part; the key sets
      * are disjoint, so the aggregates add and the grouped rows concatenate.  Single sequences only, no
-     * WHERE clause. */
+     * WHERE clause.  owner_parts = 1 (owner_part 0) keeps every k-mer: on a sequence in pieces it counts
+     * the whole sequence, on any other input it is the same as no restriction. */
     uint32_t owner_parts;
     uint32_t owner_part;
 } dnagpu_count_opts;
