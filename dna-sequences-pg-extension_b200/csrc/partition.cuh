@@ -977,11 +977,14 @@ __global__ void __launch_bounds__(kThreads) k_count_buckets(const uint64_t *__re
  * kBins sub-bins by an independent hash with a RETURNING shared-memory add (11.6 lane-ops/clk/SM
  * against 3.1 for the 64-bit CAS of the table, profiles/r01e_microbench); the value returned is the
  * key's rank r inside its bin.  Each warp scans the counts of its own bins with shuffles, the keys
- * are placed bin by bin into a staging area with their rank beside them, and every staged key is
- * compared with the r keys placed before it in its bin (r > 0 for about one key in four; the first
- * three look-backs are branch-free):
+ * are placed bin by bin into a staging area (slot = start of the bin + r), and every staged key is
+ * compared with the slots before it (the first three branch-free; further ones, up to the bin's start,
+ * only when the third holds a key of its bin):
  *     e = earlier keys equal to mine;  repeats += (e >= 1);  second += (e == 1);
  *     distinct = keys - repeats;  unique = distinct - second  (unique iff no second occurrence).
+ * No rank is stored for the compare: the bin and the bucket are both functions of the key, so a slot
+ * outside my bin -- another bin, another warp's region, or a stale key of an earlier bucket -- never
+ * holds a key equal to mine, and looking back past the start of the bin cannot change e.
  * No probe chains, no 48 KB table to clear, three barriers per bucket.  The kernel is bound by issue
  * slots, so it is written as straight-line code: lanes past the end of a bucket work on dummy bins and
  * slots, and the rank / place / load phases are instantiated per number of key rows (BINS_DISPATCH).
@@ -1024,14 +1027,12 @@ __device__ __forceinline__ void bins_load(uint64_t (&x)[kBinPer], const uint64_t
 
 template <int ROWS>
 __device__ __forceinline__ void bins_place(const uint64_t (&x)[kBinPer], const uint32_t (&f)[kBinPer / 2],
-                                           const uint16_t *st, uint64_t *stage, uint8_t *rank_at)
+                                           const uint16_t *st, uint64_t *stage)
 {
 #pragma unroll
     for (int u = 0; u < ROWS; ++u) {
         const uint32_t v = (u & 1) ? (f[u >> 1] >> 16) : (f[u >> 1] & 0xffffu);
-        const uint32_t pos = st[v & 0xfffu] + (v >> 12);
-        stage[pos] = x[u];
-        rank_at[pos] = (uint8_t)(v >> 12);
+        stage[st[v & 0xfffu] + (v >> 12)] = x[u];
     }
 }
 
@@ -1065,15 +1066,19 @@ __global__ void __launch_bounds__(kThreads, 4) k_count_buckets_bins(const uint64
     }
     /* every array ends in dummy entries, one per lane (+ 15 for a dummy's meaningless 4-bit rank): the lanes
      * past the end of a bucket's last row work on those instead of branching around the atomics and the stores */
-    __shared__ __align__(16) uint64_t stage_raw[4 + kBinCap + 48]; /* 4 in front: the compare phase looks back */
+    /* 4 slots in front: the compare phase looks back 3.  The dummy slots stage[kBinCap ..] hold whatever the lanes
+     * past the end of a bucket place there; the compare phase reads only slots before base + wtotal <= kBinCap. */
+    __shared__ __align__(16) uint64_t stage_raw[4 + kBinCap + 48];
     uint64_t *const stage = stage_raw + 4;
     __shared__ __align__(16) uint32_t cnt[kBins + 32];
-    __shared__ __align__(16) uint16_t st[kBins + 32];       /* start of the bin in `stage` */
-    __shared__ __align__(16) uint8_t rank_at[kBinCap + 48]; /* rank of the key at a stage position inside its bin */
+    __shared__ __align__(16) uint16_t st[kBins + 32]; /* start of the bin in `stage` */
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     uint32_t repeats = 0, second = 0; /* keys with >= 1 / exactly 1 equal key before them in their bin */
     unsigned long long placed = 0;    /* thread 0: keys of the buckets counted here */
     for (int i = tid; i < kBins + 32; i += kThreads) cnt[i] = 0;
+    /* kEmpty never reaches a bucket ('G' x 32 is counted on the side), so a slot never written since the launch
+     * never equals a key: the look-back may read it */
+    for (int i = tid; i < 4 + kBinCap + 48; i += kThreads) stage_raw[i] = kEmpty;
     if (tid < 32) st[kBins + tid] = (uint16_t)(kBinCap + tid);
     uint64_t b = blockIdx.x;
     uint32_t n = 0;
@@ -1101,11 +1106,14 @@ __global__ void __launch_bounds__(kThreads, 4) k_count_buckets_bins(const uint64
             /* A: rank of every key inside its bin */
             BINS_DISPATCH(n, bins_rank<ROWS>(x, f, n, tid, lane, cnt));
             __syncthreads();
-            /* B: the owner of 8 consecutive bins reads their counts and clears them; warp scan -> starts */
-            const uint4 c0 = *reinterpret_cast<const uint4 *>(&cnt[8 * tid]);
-            const uint4 c1 = *reinterpret_cast<const uint4 *>(&cnt[8 * tid + 4]);
-            *reinterpret_cast<uint4 *>(&cnt[8 * tid]) = make_uint4(0, 0, 0, 0);
-            *reinterpret_cast<uint4 *>(&cnt[8 * tid + 4]) = make_uint4(0, 0, 0, 0);
+            /* B: the owner of the bins 4 tid .. 4 tid + 3 and kBins / 2 + 4 tid .. + 3 (a 16-byte lane stride: no
+             * bank conflict) reads their counts and clears them; warp scan -> starts.  Warp w's region of the stage
+             * holds its bins 128 w .. 128 w + 127 and kBins / 2 + 128 w .. in thread order. */
+            uint32_t *const cnt_lo = &cnt[4 * tid], *const cnt_hi = &cnt[kBins / 2 + 4 * tid];
+            const uint4 c0 = *reinterpret_cast<const uint4 *>(cnt_lo);
+            const uint4 c1 = *reinterpret_cast<const uint4 *>(cnt_hi);
+            *reinterpret_cast<uint4 *>(cnt_lo) = make_uint4(0, 0, 0, 0);
+            *reinterpret_cast<uint4 *>(cnt_hi) = make_uint4(0, 0, 0, 0);
             const uint32_t s1 = c0.x, s2 = s1 + c0.y, s3 = s2 + c0.z, s4 = s3 + c0.w, s5 = s4 + c1.x, s6 = s5 + c1.y,
                            s7 = s6 + c1.z, mine = s7 + c1.w;
             const uint32_t worst = max(max(max(c0.x, c0.y), max(c0.z, c0.w)), max(max(c1.x, c1.y), max(c1.z, c1.w)));
@@ -1119,13 +1127,13 @@ __global__ void __launch_bounds__(kThreads, 4) k_count_buckets_bins(const uint64
             const bool bad = wtotal > (uint32_t)kBinWarpCap || worst > (uint32_t)kBinHeavy;
             const uint32_t p = warp * kBinWarpCap + inc - mine;
             /* (harmless when bad: the bucket is passed on and st is not read) */
-            *reinterpret_cast<uint4 *>(&st[8 * tid]) =
-                make_uint4(p | ((p + s1) << 16), (p + s2) | ((p + s3) << 16), (p + s4) | ((p + s5) << 16),
-                           (p + s6) | ((p + s7) << 16));
+            *reinterpret_cast<uint2 *>(&st[4 * tid]) = make_uint2(p | ((p + s1) << 16), (p + s2) | ((p + s3) << 16));
+            *reinterpret_cast<uint2 *>(&st[kBins / 2 + 4 * tid]) =
+                make_uint2((p + s4) | ((p + s5) << 16), (p + s6) | ((p + s7) << 16));
             pass_on = __syncthreads_or(bad);
             if (!pass_on) {
-                /* C: place, and leave the rank beside the key */
-                BINS_DISPATCH(n, bins_place<ROWS>(x, f, st, stage, rank_at));
+                /* C: place */
+                BINS_DISPATCH(n, bins_place<ROWS>(x, f, st, stage));
                 if (tid == 0) placed += n;
             }
         }
@@ -1134,17 +1142,18 @@ __global__ void __launch_bounds__(kThreads, 4) k_count_buckets_bins(const uint64
         if (n <= kBinCap) { /* uniform: the barriers above were taken */
             __syncthreads();
             if (!pass_on) {
-                /* D: a key of rank r against the r keys placed before it in its bin.  A warp walks the
-                 * region of its own bins: ranks > 0 are one in four, their loops one or two steps. */
+                /* D: a key against the keys placed before it in its bin.  A warp walks the region of its own
+                 * bins; a slot outside the bin never equals the key, so it needs no bound. */
                 const uint32_t base = warp * kBinWarpCap;
                 for (uint32_t q = base + lane; q < base + wtotal; q += 32) {
-                    /* three look-backs without a branch (rank > 3 is rare): neighbouring lanes read
-                     * neighbouring slots, and a slot before the bin is simply not counted */
-                    const uint32_t r = rank_at[q];
+                    /* three look-backs without a branch: neighbouring lanes read neighbouring slots */
                     const uint64_t key = stage[q], k1 = stage[q - 1], k2 = stage[q - 2], k3 = stage[q - 3];
-                    uint32_t e = (uint32_t)((r >= 1) & (k1 == key)) + (uint32_t)((r >= 2) & (k2 == key)) +
-                                 (uint32_t)((r >= 3) & (k3 == key));
-                    if (r > 3) { /* rare: kept out of line (the rolled loop's set-up was 13 % of the kernel's instructions, ncu r02c) */
+                    uint32_t e = (uint32_t)(k1 == key) + (uint32_t)(k2 == key) + (uint32_t)(k3 == key);
+                    const uint32_t bin = bin_of(key);
+                    if (bin_of(k3) == bin) { /* rare (rank >= 3): kept out of line (the rolled loop's set-up was 13 % of the kernel's instructions, ncu r02c) */
+                        /* the rank from the bin's start, which phase B left in st (walking on while the slots
+                         * hold keys of the bin measured 2 % slower at k = 14, where many k-mers repeat) */
+                        const uint32_t r = q - st[bin];
 #pragma unroll 1
                         for (uint32_t j = 4; j <= r; ++j) e += stage[q - j] == key;
                     }
